@@ -6,7 +6,7 @@ Workload (BASELINE.json configs[1]): SMORE on a synthetic Amazon-Baby-shaped dat
 train batch 2048, the reference trainer's mirror-gradient schedule). One "step" = one iteration of
 Trainer._train_epoch's batch loop: in steady state 3 forward+backward passes and 2 Adam steps.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 * `value`   : training interactions/s over all ranks, device-timed (CUDA events, max over ranks)
               with the K batches already resident in HBM.
@@ -26,6 +26,9 @@ Trainer._train_epoch's batch loop: in steady state 3 forward+backward passes and
               (SMORE / Clothing d = 128 with item-range sharded feature tables).
 * --impl reference : the reference's CPU implementation of the same step (oracle port on torch
               CPU with all host threads), rank 0 only; builds its inputs without the product.
+* --dump-outputs DIR : after the K timed steps, rank 0 writes what the last of them handed its caller
+              (see dump_outputs) as DIR/<name>.npy. Data, parameters and batches are seeded, so two builds
+              run with the same arguments can be compared output for output.
 """
 import argparse
 import importlib
@@ -158,6 +161,35 @@ def take_batches(loader, n):
                 loader.pr = 0
                 break
     return out
+
+
+DUMP_MAX_BYTES = 64 << 20       # whole dump
+DUMP_MAX_ELEMS = 1 << 20        # one array; a larger parameter is cut to a sample of its rows
+
+
+def dump_outputs(out_dir, loss, model):
+    """Write what a training step hands its caller -- the loss it returned and every parameter it
+    updated -- as float32 `<name>.npy` files (`loss.npy`, `<parameter name>.npy`) under `out_dir`.
+    A parameter of more than DUMP_MAX_ELEMS elements keeps a sample of its rows, the same in every
+    run: ascending row ids drawn by a generator seeded with 0 that is used for nothing else, so the
+    training's own random streams are not advanced."""
+    import numpy as np
+    import torch
+    arrays = {"loss": loss.detach().float().reshape(-1)}
+    for name, p in model.named_parameters():
+        t = p.detach()
+        if t.numel() > DUMP_MAX_ELEMS:
+            keep = max(1, DUMP_MAX_ELEMS * t.shape[0] // t.numel())
+            rows = np.sort(np.random.default_rng(0).choice(t.shape[0], keep, replace=False))
+            t = t[torch.from_numpy(rows).to(t.device)]
+        arrays[name] = t.float()
+    arrays = {k: v.cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte budget")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 def time_kernel(fn, flush, iters=20, warm=3):
@@ -347,7 +379,7 @@ def run_ours(args):
     torch.cuda.nvtx.range_push("timed_steps")          # ncu --nvtx --nvtx-include "timed_steps/"
     e0.record()
     for b in batches[W:]:
-        trainer._train_batch_graphed(b)
+        loss = trainer._train_batch_graphed(b)
     e1.record()
     torch.cuda.nvtx.range_pop()
     barrier()
@@ -358,6 +390,8 @@ def run_ours(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     value = world * K * B / (ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, model)     # before the end-to-end epochs train on
 
     # ---- end to end through the public API: loader (host sampling, pinned H2D) + loss D2H
     # Trainer._train_epoch with the reference's per-batch `loss.item()` (sync_free off): every step
@@ -926,7 +960,13 @@ def main():
     ap.add_argument("--chunks", type=int, default=4)
     ap.add_argument("--no-sharded-blocks", action="store_true",
                     help="skip the config-5 / config-4 blocks of the default workload (quick runs, ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and parameters after the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "smore_baby"):
+        ap.error("--dump-outputs applies to the default workload (--impl ours --workload smore_baby)")
     if args.workload == "scaled" and args.impl == "ours":
         run_scaled(args)
     elif args.impl == "reference":

@@ -164,8 +164,11 @@ def _check_device(t):
     """Kernels are enqueued on the CURRENT device's current stream (see `stream`): a tensor that
     lives on another GPU would be dereferenced by the wrong device, so that is an error here
     (torch ops switch devices by themselves; this library asks the caller to
-    `torch.cuda.set_device` / `with torch.cuda.device(...)` first)."""
-    if t.is_cuda and t.device.index != torch.cuda.current_device():
+    `torch.cuda.set_device` / `with torch.cuda.device(...)` first). A host tensor is an error too: its
+    address would reach a kernel as a device pointer."""
+    if not t.is_cuda:
+        raise RuntimeError("mmrec_b200 operators need CUDA tensors; there is no CPU fallback")
+    if t.device.index != torch.cuda.current_device():
         raise RuntimeError(f"mmrec_b200: tensor on {t.device} but the current CUDA device is "
                            f"cuda:{torch.cuda.current_device()}; wrap the call in torch.cuda.device(tensor.device)")
 

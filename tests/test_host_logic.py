@@ -355,3 +355,31 @@ def test_epoch_shuffle_prefetch_draws_the_same_permutations(tiny_data):
                           np.random.get_state()[1].copy(), random.getstate())
     assert torch.equal(seen[False][0], seen[True][0])
     assert np.array_equal(seen[False][1], seen[True][1]) and seen[False][2] == seen[True][2]
+
+
+def test_bench_dump_outputs_is_a_seeded_float32_sample(tmp_path):
+    """bench.py --dump-outputs: the loss and every parameter as float32 .npy; a parameter above the per-array
+    limit keeps the same ascending sample of its rows on every call, and the global numpy / torch random
+    streams the training draws from are not advanced."""
+    import bench
+    model = torch.nn.Module()
+    n_rows = bench.DUMP_MAX_ELEMS // 8 + 3
+    model.big = torch.nn.Parameter(torch.arange(n_rows, dtype=torch.float32).repeat_interleave(8).reshape(n_rows, 8))
+    model.small = torch.nn.Linear(3, 2).double()
+    np.random.seed(5)
+    torch.manual_seed(5)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), torch.tensor(1.5), model)
+    assert np.random.randint(1 << 30) == np.random.RandomState(5).randint(1 << 30)
+    assert torch.equal(torch.rand(4), torch.rand(4, generator=torch.Generator().manual_seed(5)))
+    names = {"loss.npy", "big.npy", "small.weight.npy", "small.bias.npy"}
+    assert set(os.listdir(tmp_path / "a")) == names
+    for f in names:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype == np.float32 and np.array_equal(a, b)
+    assert np.load(tmp_path / "a" / "loss.npy").tolist() == [1.5]
+    assert np.array_equal(np.load(tmp_path / "a" / "small.weight.npy"), model.small.weight.detach().float().numpy())
+    big = np.load(tmp_path / "a" / "big.npy")
+    assert big.size <= bench.DUMP_MAX_ELEMS and big.shape[1] == 8
+    rows = big[:, 0]
+    assert np.all(np.diff(rows) > 0) and rows[-1] < n_rows and np.array_equal(big, np.repeat(rows[:, None], 8, 1))
