@@ -160,6 +160,33 @@ int mmrec_bpr_bwd_f32(const float *user_emb, const float *item_emb, int32_t d,
                       void *stream);
 
 /* ------------------------------------------------------------------------------------------
+ * LightGCN loss (lightgcn.py:133-159: BPRLoss with gamma + EmbLoss) on any subset of a batch's
+ * triples, e.g. the triples one rank of a user-sharded run owns. `users` index the user tables
+ * (shard-local rows), `pos` / `neg` the item tables; batch may be 0.
+ *   x_b = <uo_b, po_b> - <uo_b, no_b>   (final tables user_out / item_out)
+ *   out4 = (sum_b -log(gamma + sigmoid(x_b)), sum_b |u0_b|^2, sum_b |p0_b|^2, sum_b |n0_b|^2)
+ *          (u0 / p0 / n0: rows of the ego tables user_ego / item_ego), reduced in a fixed order;
+ *   dx[b] = d(-log(gamma + sigmoid(x)))/dx at x_b  (saved for the backward).
+ * The caller reduces out4 (across ranks), forms the loss and the coefficients
+ *   coef4 = (1/B, reg/(B |U|), reg/(B |P|), reg/(B |N|))  (device scalars; B and the norms global)
+ * and the backward scatter-adds (atomics, duplicates allowed) into four zeroed outputs:
+ *   d_user_out[u_b] += c0 dx_b (po_b - no_b); d_item_out[p_b] += c0 dx_b uo_b; d_item_out[n_b] -= c0 dx_b uo_b;
+ *   d_user_ego[u_b] += c1 u0_b; d_item_ego[p_b] += c2 p0_b; d_item_ego[n_b] += c3 n0_b.
+ * d % 4 == 0, tables 16-byte aligned; partial holds
+ * mmrec_lightgcn_loss_fwd_workspace_floats(batch) floats; counter one zero-initialised uint32.
+ * ---------------------------------------------------------------------------------------- */
+size_t mmrec_lightgcn_loss_fwd_workspace_floats(int32_t batch);
+int mmrec_lightgcn_loss_fwd_f32(const float *user_out, const float *item_out, const float *user_ego,
+                                const float *item_ego, int32_t d, const int64_t *users, const int64_t *pos,
+                                const int64_t *neg, int32_t batch, float gamma, float *out4, float *dx,
+                                float *partial, uint32_t *counter, void *stream);
+int mmrec_lightgcn_loss_bwd_f32(const float *user_out, const float *item_out, const float *user_ego,
+                                const float *item_ego, int32_t d, const int64_t *users, const int64_t *pos,
+                                const int64_t *neg, int32_t batch, const float *dx, const float *coef4,
+                                float *d_user_out, float *d_item_out, float *d_user_ego, float *d_item_ego,
+                                void *stream);
+
+/* ------------------------------------------------------------------------------------------
  * InfoNCE (K7). Replaces MGCN/SMORE.InfoNCE (mgcn.py:224-231, smore.py:380-387).
  *   v1 = normalize(T1[idx]), v2 = normalize(T2[idx]) (F.normalize, eps 1e-12)
  *   loss = mean_i( -log( exp(<v1_i,v2_i>/t) / sum_j exp(<v1_i,v2_j>/t) ) )

@@ -228,15 +228,50 @@ class DeviceTrainLoader:
     same sampling rule (uniform item, rejected while in the user's training history) on the
     stateless counter stream of mmrec_neg_sample_counter, so every rank of a sharded run can
     regenerate exactly the same batch from (seed, epoch, batch index) without a broadcast.
-    `users` / `items`: the training interactions on the device (int64)."""
+    `users` / `items`: the training interactions on the device (int64).
 
-    def __init__(self, users, items, n_users, n_items, batch_size, seed=999, shuffle=True, max_draws=64):
+    Per-rank batches (`rank` given; for a user-sharded model such as parallel.ShardedLightGCN):
+    `users` / `items` are this rank's interactions only, its users [user_lo, user_lo + n_users);
+    batches carry LOCAL user ids (global - user_lo) and negatives come from a history CSR over the
+    local users, on the counter stream of seed `rank_seed(seed, rank)`. One all-gather of the ranks'
+    interaction counts at set-up (the world size is the process group's) fixes the number of steps S = ceil(E_total / batch_size) on every
+    rank; a rank's shuffled interactions are cut into exactly S slices of near-equal size (they
+    differ by at most one, some are empty when the rank holds fewer than S interactions), so every
+    rank runs the same collectives. The global batch of a step is the union of the ranks' slices.
+    `pr` counts steps in this mode. `sampler` replaces the CUDA sampler with a callable of
+    oracle.sampler.neg_sample_counter's arguments (users, all_items=None, n_items, hist_rowptr,
+    hist_cols, seed, step, max_draws) -> negatives; then host tensors are accepted."""
+
+    def __init__(self, users, items, n_users, n_items, batch_size, seed=999, shuffle=True, max_draws=64,
+                 rank=None, world=None, user_lo=0, group=None, sampler=None):
         from . import lib
-        lib.require_cuda(users, items)
+        if sampler is None:
+            lib.require_cuda(users, items)
+        self.sampler = sampler
         self.users, self.items = users.to(torch.int64).contiguous(), items.to(torch.int64).contiguous()
         self.n_users, self.n_items, self.step = int(n_users), int(n_items), int(batch_size)
         self.seed, self.shuffle, self.max_draws = int(seed), bool(shuffle), int(max_draws)
         self.device = users.device
+        self.rank = rank
+        if rank is not None:
+            import torch.distributed as dist
+            if dist.is_available() and dist.is_initialized():
+                # S must come from every rank's count: a world size that disagrees with the group
+                # would give ranks different step counts and hang the collectives of the last steps
+                pg_world = dist.get_world_size(group)
+                if world is not None and int(world) != pg_world:
+                    raise ValueError(f"DeviceTrainLoader: world={world} but the process group has {pg_world} ranks")
+                world = pg_world
+            elif world not in (None, 1):
+                raise ValueError("DeviceTrainLoader: world > 1 needs an initialised process group")
+            world = 1 if world is None else int(world)
+            self.users = self.users - int(user_lo)
+            self.seed = rank_seed(seed, rank)
+            self.nnz_per_rank = [int(self.users.numel())]
+            if world > 1:
+                self.nnz_per_rank = [None] * world
+                dist.all_gather_object(self.nnz_per_rank, int(self.users.numel()), group=group)
+            self.n_steps = -(-sum(self.nnz_per_rank) // self.step)
         # per-user history CSR, ascending item ids (the rejection test is a binary search)
         key = torch.sort(self.users * self.n_items + self.items)[0]
         self.hist_cols = (key % self.n_items).to(torch.int32).contiguous()
@@ -248,24 +283,34 @@ class DeviceTrainLoader:
         self.order = None
 
     def __len__(self):
+        if self.rank is not None:
+            return self.n_steps
         return -(-self.users.numel() // self.step)
 
     def __iter__(self):
         self.epoch += 1
         self.pr = 0
         if self.shuffle:
-            g = torch.Generator(device=self.device).manual_seed(self.seed + self.epoch)
+            g = torch.Generator(device=self.device).manual_seed((self.seed + self.epoch) & 0xFFFFFFFFFFFFFFFF)
             self.order = torch.randperm(self.users.numel(), generator=g, device=self.device)
         return self
 
     def sample_negatives(self, u, step_id):
         from . import lib
+        if u.numel() == 0:             # an empty per-rank slice: nothing to draw (the C ABI rejects NULL operands)
+            return torch.empty_like(u)
+        if self.sampler is not None:
+            neg = self.sampler(u.cpu().numpy(), None, self.n_items, self.hist_rowptr.cpu().numpy(),
+                               self.hist_cols.cpu().numpy(), self.seed, int(step_id), self.max_draws)
+            return torch.as_tensor(neg, dtype=torch.int64).to(u.device)
         neg = torch.empty_like(u)
         lib.call("mmrec_neg_sample_counter", lib.ptr(u), u.numel(), None, self.n_items, lib.ptr(self.hist_rowptr),
                  lib.ptr(self.hist_cols), self.seed, int(step_id), self.max_draws, lib.ptr(neg), lib.stream())
         return neg
 
     def __next__(self):
+        if self.rank is not None:
+            return self._next_rank_slice()
         if self.pr >= self.users.numel():
             raise StopIteration
         sl = slice(self.pr, self.pr + self.step)
@@ -275,6 +320,21 @@ class DeviceTrainLoader:
         step_id = self.epoch * len(self) + self.pr // self.step
         self.pr += self.step
         return torch.stack([u, i, self.sample_negatives(u, step_id)])
+
+    def _next_rank_slice(self):
+        s, S, n = self.pr, self.n_steps, self.users.numel()
+        if s >= S:
+            raise StopIteration
+        a, b = s * n // S, (s + 1) * n // S
+        idx = self.order[a:b] if self.order is not None else torch.arange(a, b, device=self.device)
+        u, i = self.users[idx].contiguous(), self.items[idx]
+        self.pr += 1
+        return torch.stack([u, i, self.sample_negatives(u, self.epoch * S + s)])
+
+
+def rank_seed(seed, rank):
+    """Sampler / shuffle seed of rank `rank` in per-rank batching (rank 0 keeps `seed`)."""
+    return (int(seed) ^ (int(rank) * 0x9E3779B97F4A7C15)) & 0xFFFFFFFFFFFFFFFF
 
 
 class EvalDataLoader(AbstractDataLoader):

@@ -35,6 +35,9 @@ SIGNATURES = {
     "mmrec_layergcn_cos_bwd_f32": (C.c_int, [_p, _p, _p, _p, _i32, _i32, _p, _p, _p]),
     "mmrec_bpr_fwd_f32": (C.c_int, [_p, _p, _i32, _p, _p, _p, _i32, _p, _p, _p, _p, _p]),
     "mmrec_bpr_bwd_f32": (C.c_int, [_p, _p, _i32, _p, _p, _p, _i32, _p, _p, _p, _p, _p]),
+    "mmrec_lightgcn_loss_fwd_workspace_floats": (_sz, [_i32]),
+    "mmrec_lightgcn_loss_fwd_f32": (C.c_int, [_p, _p, _p, _p, _i32, _p, _p, _p, _i32, _f32, _p, _p, _p, _p, _p]),
+    "mmrec_lightgcn_loss_bwd_f32": (C.c_int, [_p, _p, _p, _p, _i32, _p, _p, _p, _i32, _p, _p, _p, _p, _p, _p, _p]),
     "mmrec_infonce_splits": (_i32, [_i32]),
     "mmrec_infonce_fwd_workspace_floats": (_sz, [_i32]),
     "mmrec_infonce_fwd_f32": (C.c_int, [_p, _p, _i32, _p, _i32, _f32, _p, _p, _p, _p, _p, _p, _p,

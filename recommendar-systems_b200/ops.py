@@ -390,6 +390,62 @@ def bpr_table(all_emb, n_users, users, pos, neg):
     return _BPRTable.apply(all_emb, n_users, users, pos, neg)
 
 
+# ------------------------------------------------------------------------------- LightGCN loss
+def _lightgcn_loss_args(what, user_out, item_out, user_ego, item_ego, users, pos, neg):
+    """Checks shared by the forward and the backward: float32 CUDA tables of matching shapes,
+    int64 CUDA ids of one length inside their tables (range checked with MMREC_CHECK_IDS=1)."""
+    user_out, item_out, user_ego, item_ego = (_f32c(t) for t in (user_out, item_out, user_ego, item_ego))
+    lib.require_cuda(user_out, item_out, user_ego, item_ego, users, pos, neg)
+    B, d = users.numel(), user_out.shape[1]
+    if pos.numel() != B or neg.numel() != B or users.dtype != torch.int64 or pos.dtype != torch.int64 \
+            or neg.dtype != torch.int64:
+        raise RuntimeError(f"{what}: users / pos / neg must be int64 tensors of one length")
+    if not (item_out.shape[1] == user_ego.shape[1] == item_ego.shape[1] == d) or \
+            user_ego.shape[0] != user_out.shape[0] or item_ego.shape[0] != item_out.shape[0]:
+        raise RuntimeError(f"{what}: final and ego tables must have matching shapes")
+    _check_ids(users, user_out.shape[0], f"{what} users")
+    _check_ids(pos, item_out.shape[0], f"{what} positive items")
+    _check_ids(neg, item_out.shape[0], f"{what} negative items")
+    return user_out, item_out, user_ego, item_ego, users.contiguous(), pos.contiguous(), neg.contiguous()
+
+
+def lightgcn_loss_fwd(user_out, item_out, user_ego, item_ego, users, pos, neg, gamma=1e-10):
+    """Partial sums of LightGCN's loss (lightgcn.py:133-159) over these triples (no autograd):
+    -> (out4 = [sum -log(gamma + sigmoid(x)), sum |u0|^2, sum |p0|^2, sum |n0|^2], dx [B]);
+    `users` index the user tables, `pos` / `neg` the item tables (int64; B may be 0)."""
+    user_out, item_out, user_ego, item_ego, users, pos, neg = _lightgcn_loss_args(
+        "lightgcn_loss_fwd", user_out, item_out, user_ego, item_ego, users, pos, neg)
+    B, d = users.numel(), user_out.shape[1]
+    dev = user_out.device
+    out4 = torch.empty(4, dtype=torch.float32, device=dev)
+    dx = torch.empty(B, dtype=torch.float32, device=dev)
+    partial = torch.empty(lib.load().mmrec_lightgcn_loss_fwd_workspace_floats(B), dtype=torch.float32, device=dev)
+    lib.call("mmrec_lightgcn_loss_fwd_f32", lib.ptr(user_out), lib.ptr(item_out), lib.ptr(user_ego),
+             lib.ptr(item_ego), d, lib.ptr(users), lib.ptr(pos), lib.ptr(neg), B, float(gamma), lib.ptr(out4),
+             lib.ptr(dx), lib.ptr(partial), lib.ptr(_counter(dev)), lib.stream())
+    return out4, dx
+
+
+def lightgcn_loss_bwd(user_out, item_out, user_ego, item_ego, users, pos, neg, dx, coef4,
+                      d_user_out, d_item_out, d_user_ego, d_item_ego):
+    """Scatter-adds the gradients of the loss formed from `lightgcn_loss_fwd`'s sums into the four
+    zeroed float32 outputs (shapes of the four tables). coef4 (device float32 [4]) =
+    (dL/d sum_bpr, dL/d|U| / |U|, dL/d|P| / |P|, dL/d|N| / |N|), see include/mmrec_b200.h."""
+    user_out, item_out, user_ego, item_ego, users, pos, neg = _lightgcn_loss_args(
+        "lightgcn_loss_bwd", user_out, item_out, user_ego, item_ego, users, pos, neg)
+    outs = (d_user_out, d_item_out, d_user_ego, d_item_ego)
+    lib.require_cuda(dx, coef4, *outs)
+    for o, t in zip(outs, (user_out, item_out, user_ego, item_ego)):
+        if o.shape != t.shape or o.dtype != torch.float32 or not o.is_contiguous():
+            raise RuntimeError("lightgcn_loss_bwd: outputs must be contiguous float32 tensors shaped like the tables")
+    if dx.dtype != torch.float32 or dx.numel() != users.numel() or coef4.numel() != 4:
+        raise RuntimeError("lightgcn_loss_bwd: dx must be float32 [B] (from lightgcn_loss_fwd), coef4 [4]")
+    lib.call("mmrec_lightgcn_loss_bwd_f32", lib.ptr(user_out), lib.ptr(item_out), lib.ptr(user_ego),
+             lib.ptr(item_ego), user_out.shape[1], lib.ptr(users), lib.ptr(pos), lib.ptr(neg), users.numel(),
+             lib.ptr(dx.contiguous()), lib.ptr(_f32c(coef4)), lib.ptr(d_user_out), lib.ptr(d_item_out),
+             lib.ptr(d_user_ego), lib.ptr(d_item_ego), lib.stream())
+
+
 # ------------------------------------------------------------------------------------- InfoNCE
 class _InfoNCEPair(torch.autograd.Function):
     """cl_items + cl_users of MGCN/SMORE.calculate_loss (mgcn.py:248-251, smore.py:403-408) on

@@ -276,10 +276,18 @@ class ShardedBipartite:
 
 @torch.no_grad()
 def bipartite_propagate_mean(sb: ShardedBipartite, Xu_local, Xi, n_layers, group=None, spmm_fn=_spmm_cuda,
-                             chunks=4, timing=None):
+                             chunks=4, timing=None, reduce_items=False, after_first_exchange=None):
     """mean_{l=0..L} A^l X0 for a bipartite graph, users sharded / items replicated.
     Xu_local [hi - lo, d]: this rank's user rows of X0; Xi [I, d]: the item rows (same on every
     rank). Returns (users' rows of this rank, all item rows).
+    reduce_items=True: Xi is this rank's PARTIAL of the item rows (the backward, where each rank
+    holds the item gradient of its own triples); their sum over the group is the operand. Its
+    chunked all-reduce is issued first and waited for like a layer's yi: (a) of layer 1 runs under
+    it, (b) of layer 1 waits.
+    after_first_exchange: called once, right after layer 1's item-table all-reduce is issued, to
+    queue another collective on the group's stream behind the exchanges issued so far (with
+    reduce_items: the operand's and layer 1's), so that it runs under (b) of layer 1 and (a) of
+    layer 2 instead of delaying the operand's reduction that (b) of layer 1 waits for.
 
     Per layer l a rank computes (a) what its users add to every item, yi_l = R_p^T xu_{l-1}, and
     (b) its users' rows, yu_l = R_p xi_{l-1}; the only exchange is the all-reduce of yi_l. The item
@@ -291,15 +299,20 @@ def bipartite_propagate_mean(sb: ShardedBipartite, Xu_local, Xi, n_layers, group
     4 I d all-reduce, so the exchange hides completely while it is the shorter of the two.
     `timing` (dict of lists of (start, end) CUDA events per phase) is filled when given."""
     L = n_layers
+    multi = sb.world > 1
     if L == 0:
-        return Xu_local.clone(), Xi.clone()
+        xi0 = Xi.clone()
+        if reduce_items and multi:
+            dist.all_reduce(xi0, group=group)
+        if after_first_exchange is not None:
+            after_first_exchange()
+        return Xu_local.clone(), xi0
     scale = 1.0 / (L + 1)
     acc_u, acc_i = Xu_local, Xi.clone()
     xu, xi = Xu_local.contiguous(), Xi.contiguous()
     d = xi.shape[1]
     blocked = getattr(sb, "Rt_blocked", None)
     parts = sb.rt_chunks(chunks) if blocked is None else None
-    multi = sb.world > 1
 
     def mark(name):
         if timing is None:
@@ -314,6 +327,13 @@ def bipartite_propagate_mean(sb: ShardedBipartite, Xu_local, Xi, n_layers, group
             ev[1].record()
 
     pending = None                                            # (works, yi) of the previous layer
+    if reduce_items:
+        xi = acc_i                                            # reduced in place; read by (b) of layer 1 only
+        works = []
+        if multi:
+            ranges = [(0, sb.I)] if parts is None else [(a, b) for _, a, b in parts]
+            works = [dist.all_reduce(acc_i[a:b], group=group, async_op=True) for a, b in ranges]
+        pending = (works, None)
     for l in range(1, L + 1):
         last = l == L
         yi = torch.empty(sb.I, d, dtype=xi.dtype, device=xi.device)
@@ -337,13 +357,16 @@ def bipartite_propagate_mean(sb: ShardedBipartite, Xu_local, Xi, n_layers, group
                 if multi:
                     works.append(dist.all_reduce(yi[a:b], group=group, async_op=True))
         done(ev)
+        if l == 1 and after_first_exchange is not None:
+            after_first_exchange()
         if pending is not None:                               # (b) needs the reduced item table of layer l - 1
             ev = mark("exposed_all_reduce")
             for w in pending[0]:
                 w.wait()
             done(ev)
-            acc_i.add_(pending[1])
-            xi = pending[1]
+            if pending[1] is not None:
+                acc_i.add_(pending[1])
+                xi = pending[1]
         yu = None if last else torch.empty_like(xu)
         acc_new = torch.empty_like(xu)
         ev = mark("r_spmm")
@@ -376,6 +399,198 @@ def bipartite_score_topk(sb: ShardedBipartite, out_u_local, out_i, users, k, gro
     rows = torch.arange(users.numel(), device=users.device)
     return sharded_score_topk(ub, rows, out_i[lo:hi].contiguous(), lo, k, group=group, local_topk=local_topk,
                               merge=merge)
+
+
+# ------------------------------------------------------------------ training on the user-sharded graph
+def _span(timing, name):
+    """(start, end) CUDA events of one phase, appended to timing[name]; None when not timing."""
+    if timing is None:
+        return None
+    ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
+    timing.setdefault(name, []).append(ev)
+    ev[0].record()
+    return ev
+
+
+def _end(ev):
+    if ev is not None:
+        ev[1].record()
+
+
+class _BipartitePropagateMean(torch.autograd.Function):
+    """bipartite_propagate_mean with a backward. mean_{l=0..L} A^l is symmetric, so the backward
+    is the same operator on (dU_local, dI); dI is this rank's partial (the item gradient of the
+    triples it owns) and is summed over the group by the operator's first, overlapped, exchange."""
+
+    @staticmethod
+    def forward(ctx, Xu_local, Xi, sb, n_layers, group, spmm_fn, chunks, timing, backward_exchange_hook):
+        ctx.args = (sb, n_layers, group, spmm_fn, chunks, timing, backward_exchange_hook)
+        ev = _span(timing, "forward_propagation")
+        out = bipartite_propagate_mean(sb, Xu_local.detach(), Xi.detach(), n_layers, group, spmm_fn, chunks, timing)
+        _end(ev)
+        return out
+
+    @staticmethod
+    def backward(ctx, dU, dI):
+        sb, L, group, spmm_fn, chunks, timing, hook = ctx.args
+        ev = _span(timing, "backward_propagation")
+        gu, gi = bipartite_propagate_mean(sb, dU.contiguous(), dI.contiguous(), L, group, spmm_fn, chunks, timing,
+                                          reduce_items=True, after_first_exchange=hook)
+        _end(ev)
+        return gu, gi, None, None, None, None, None, None, None
+
+
+def bipartite_propagate(sb: ShardedBipartite, Xu_local, Xi, n_layers, group=None, spmm_fn=_spmm_cuda, chunks=4,
+                        timing=None, backward_exchange_hook=None):
+    """Differentiable bipartite_propagate_mean. Backward exchanges: one chunked all-reduce of the
+    partial item gradient, then one per layer as in the forward (1 + L); the returned item
+    gradient is the group's total, identical on every rank. `backward_exchange_hook` is the
+    backward's `after_first_exchange` (see bipartite_propagate_mean)."""
+    return _BipartitePropagateMean.apply(Xu_local, Xi, sb, n_layers, group, spmm_fn, chunks, timing,
+                                         backward_exchange_hook)
+
+
+def _xavier_rows(n, d, lo, hi, seed, device):
+    """Rows [lo, hi) of an xavier-uniform [n, d] table (fan n + d, models.LightGCN's init),
+    generated in fixed 1M-row blocks so the values do not depend on how the rows are sharded."""
+    bound = (6.0 / (n + d)) ** 0.5
+    blk = 1 << 20
+    out = [torch.empty(0, d, device=device)]
+    for b0 in range(lo // blk * blk, hi, blk):
+        b1 = min(n, b0 + blk)
+        g = torch.Generator(device=device).manual_seed(seed + b0 // blk)
+        x = (torch.rand(b1 - b0, d, generator=g, device=device) * 2 - 1) * bound
+        out.append(x[max(lo, b0) - b0: min(hi, b1) - b0])
+    return torch.cat(out).contiguous()
+
+
+def _loss_fns_cuda():
+    return ops.lightgcn_loss_fwd, ops.lightgcn_loss_bwd
+
+
+class _ShardedLightGCNLoss(torch.autograd.Function):
+    """LightGCN's loss over the union of every rank's triples from this rank's share: partial sums
+    on the local triples, one all-reduce of [bpr, |U|^2, |P|^2, |N|^2, B_p], the global loss and the
+    backward coefficients formed on the device (no host round trip)."""
+
+    @staticmethod
+    def forward(ctx, user_out, item_out, user_ego, item_ego, users, pos, neg, model):
+        fwd, _ = model.loss_fns
+        ev = _span(model.timing, "loss")
+        out4, dx = fwd(user_out.detach(), item_out.detach(), user_ego.detach(), item_ego.detach(), users, pos, neg,
+                       model.gamma)
+        # B_p travels with the sums (exact in float32 up to 2^24 triples per step)
+        red = torch.cat([out4, out4.new_full((1,), float(users.numel()))])
+        if model.sb.world > 1:
+            dist.all_reduce(red, group=model.group)
+        B = red[4].clamp(min=1.0)
+        norms = red[1:4].sqrt()
+        rw = model.reg_weight
+        loss = red[0] / B + rw * (norms.sum() / B)
+        # d|x|/dx = x / |x|, and 0 at x = 0 as torch.norm's backward
+        reg = torch.where(norms > 0, rw / (B * norms.clamp(min=torch.finfo(norms.dtype).tiny)),
+                          torch.zeros_like(norms))
+        ctx.coef4 = torch.cat([(1.0 / B).reshape(1), reg]).to(out4.dtype)
+        ctx.model = model
+        ctx.save_for_backward(user_out, item_out, user_ego, item_ego, users, pos, neg, dx)
+        _end(ev)
+        return loss
+
+    @staticmethod
+    def backward(ctx, g):
+        user_out, item_out, user_ego, item_ego, users, pos, neg, dx = ctx.saved_tensors
+        model = ctx.model
+        _, bwd = model.loss_fns
+        ev = _span(model.timing, "loss")
+        grads = [torch.zeros_like(t) for t in (user_out, item_out, user_ego, item_ego)]
+        bwd(user_out, item_out, user_ego, item_ego, users, pos, neg, dx, ctx.coef4 * g, *grads)
+        _end(ev)
+        model._hold_item_reg_grad(grads[3])
+        return grads[0], grads[1], grads[2], None, None, None, None, None
+
+
+class ShardedLightGCN(torch.nn.Module):
+    """LightGCN (lightgcn.py, the reference's loss semantics) trained on the user-sharded bipartite
+    graph: rank p holds the ego rows of its users [lo, hi) and the whole (replicated) item table;
+    `sb` is its ShardedBipartite (e.g. from `ShardedBipartite.from_local_edges`).
+
+    Per step: L item-table all-reduces in the forward propagation, one scalar all-reduce of the loss
+    sums, 1 + L in the backward propagation and one of the item-table regulariser gradient. The
+    latter is queued on the group's stream right after the backward's layer-1 exchange (behind the
+    reduction of the partial item gradient that layer 1 waits for, not in front of it) and waited
+    for when the item table's gradient is complete (just before the optimizer step). The item table and its optimizer state stay bit-identical on every
+    rank: every operation after a reduction runs on replicated, reduced values in a fixed order.
+
+    `user_emb` / `item_emb`: initial tables (this rank's user rows, all item rows); default: xavier
+    uniform per table, from fixed seeded 1M-row blocks (the same values at every world size).
+    `spmm_fn` / `loss_fns` = (fwd, bwd) replace the CUDA operators (ops.lightgcn_loss_fwd / _bwd
+    signatures), e.g. by float64 CPU arithmetic in tests."""
+
+    def __init__(self, sb: ShardedBipartite, embedding_size=64, n_layers=4, reg_weight=1e-2, group=None,
+                 user_emb=None, item_emb=None, seed=2024, chunks=4, gamma=1e-10, spmm_fn=_spmm_cuda, loss_fns=None,
+                 device=None):
+        super().__init__()
+        self.sb, self.group, self.n_layers, self.reg_weight = sb, group, int(n_layers), float(reg_weight)
+        self.chunks, self.gamma, self.spmm_fn = chunks, float(gamma), spmm_fn
+        self.loss_fns = loss_fns or _loss_fns_cuda()
+        self.n_users, self.n_items, self.latent_dim = sb.U, sb.I, int(embedding_size)
+        dev = torch.device(device) if device is not None else sb.R.vals.device
+        if user_emb is None:
+            user_emb = _xavier_rows(sb.U, self.latent_dim, sb.lo, sb.hi, seed, dev)
+        if item_emb is None:
+            item_emb = _xavier_rows(sb.I, self.latent_dim, 0, sb.I, seed + (1 << 20), dev)
+        if user_emb.shape != (sb.hi - sb.lo, self.latent_dim) or item_emb.shape != (sb.I, self.latent_dim):
+            raise ValueError("ShardedLightGCN: user_emb must be [hi - lo, d] (this rank's rows), item_emb [I, d]")
+        self.embedding_dict = torch.nn.ParameterDict({
+            "user_emb": torch.nn.Parameter(user_emb.detach().clone().contiguous()),
+            "item_emb": torch.nn.Parameter(item_emb.detach().clone().contiguous())})
+        self.embedding_dict["item_emb"].register_post_accumulate_grad_hook(self._finish_item_grad)
+        self._pending_item_reg = None
+        self.timing = None            # dict: CUDA-event spans per phase (scripts/sharded_train.py)
+
+    def forward(self):
+        """-> (this rank's rows of the final user table, the final item table)."""
+        e = self.embedding_dict
+        return bipartite_propagate(self.sb, e["user_emb"], e["item_emb"], self.n_layers, self.group, self.spmm_fn,
+                                   self.chunks, self.timing, backward_exchange_hook=self._issue_item_reg)
+
+    def calculate_loss(self, interaction):
+        """interaction: this rank's [3, B_p] triples (users as LOCAL row ids, global item ids; B_p
+        may be 0). Returns the loss of the union of all ranks' triples, identical on every rank."""
+        users, pos, neg = interaction[0], interaction[1], interaction[2]
+        uo, io = self.forward()
+        e = self.embedding_dict
+        return _ShardedLightGCNLoss.apply(uo, io, e["user_emb"], e["item_emb"], users, pos, neg, self)
+
+    def _hold_item_reg_grad(self, d_item_ego):
+        """Loss backward: this rank's partial of the item-ego gradient; reduced by _issue_item_reg."""
+        self._pending_item_reg = {"grad": d_item_ego, "work": None, "issued": False}
+
+    def _issue_item_reg(self):
+        """Propagation backward, after its layer-1 exchange: queue the regulariser all-reduce."""
+        pend = self._pending_item_reg
+        if pend is not None and not pend["issued"]:
+            if self.sb.world > 1:
+                pend["work"] = dist.all_reduce(pend["grad"], group=self.group, async_op=True)
+            pend["issued"] = True
+
+    def _finish_item_grad(self, p):
+        """The item table's gradient is complete: add the reduced regulariser gradient."""
+        self._issue_item_reg()
+        pend, self._pending_item_reg = self._pending_item_reg, None
+        if pend is None:
+            return
+        ev = _span(self.timing, "exposed_all_reduce")
+        if pend["work"] is not None:
+            pend["work"].wait()
+        _end(ev)
+        p.grad.add_(pend["grad"])
+
+    @torch.no_grad()
+    def full_sort_topk(self, users, k):
+        """Top-k item ids (unmasked) for GLOBAL user ids `users`, the same on every rank."""
+        uo, io = self.forward()
+        return bipartite_score_topk(self.sb, uo, io, users, k, group=self.group)
 
 
 # ------------------------------------------------------------------ item-range sharded modality tables
