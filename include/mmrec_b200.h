@@ -506,6 +506,15 @@ int mmrec_score_mask_topk_simt_f32(const float *user_emb, const int64_t *users, 
                                    int32_t d, const int32_t *mask_rowptr, const int32_t *mask_cols,
                                    int32_t k, int32_t n_splits, float *ws_val, int32_t *ws_idx,
                                    float *out_val, int64_t *out_idx, void *stream);
+/* mmrec_score_mask_topk_f32 with the mask row of entry b looked up by user id: mask_rowptr[users[b]]
+ * ..mask_rowptr[users[b] + 1] index mask_cols, i.e. the mask is a CSR over the rows of user_emb
+ * (for instance a rank's training CSR in user-sharded evaluation) instead of a per-batch CSR.
+ * Same kernels (tcgen05 for d = 32 / 64 / 128 where K fits, CUDA cores otherwise), same output. */
+int mmrec_score_mask_topk_rows_f32(const float *user_emb, const int64_t *users, int32_t n_users,
+                                   const float *item_emb, int32_t n_items, int32_t item_offset,
+                                   int32_t d, const int32_t *mask_rowptr, const int32_t *mask_cols,
+                                   int32_t k, int32_t n_splits, float *ws_val, int32_t *ws_idx,
+                                   float *out_val, int64_t *out_idx, void *stream);
 /* ----------------------------------------------------------------------------------------
  * a5 -- item-item kNN modality graphs: build_sim / build_knn_normalized_graph /
  * get_sparse_laplacian (utils/utils.py:134-137, 171-184, 139-152) and FREEDOM.get_knn_adj_mat /

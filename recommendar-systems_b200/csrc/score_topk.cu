@@ -22,7 +22,7 @@ template <int D>
 __global__ void __launch_bounds__(kUsers)
 score_topk_kernel(const float *__restrict__ user_emb, const int64_t *__restrict__ users, int n_users,
                   const float *__restrict__ item_emb, int n_items, int item_offset,
-                  const int32_t *__restrict__ mask_rowptr, const int32_t *__restrict__ mask_cols,
+                  const int32_t *__restrict__ mask_rowptr, const int32_t *__restrict__ mask_cols, int mask_by_user,
                   int k, int items_per_split, float *__restrict__ ws_val, int32_t *__restrict__ ws_idx) {
   extern __shared__ __align__(16) float smem[];
   float *sV = smem;                                   // [kItemTile][D]
@@ -46,11 +46,13 @@ score_topk_kernel(const float *__restrict__ user_emb, const int64_t *__restrict_
 #pragma unroll
     for (int c = 0; c < D; ++c) u[c] = 0.f;
   }
-  // mask cursor: first train item of this user with global id >= item_offset + j_begin
+  // mask cursor: first train item of this user with global id >= item_offset + j_begin; the mask
+  // row is the batch entry b, or the user id itself (mask_by_user: a CSR over the user table)
   int mp = 0, mend = 0, next_masked = INT_MAX;
   if (live && mask_rowptr != nullptr) {
-    int lo = mask_rowptr[b];
-    mend = mask_rowptr[b + 1];
+    const int mrow = mask_by_user ? (int)users[b] : b;
+    int lo = mask_rowptr[mrow];
+    mend = mask_rowptr[mrow + 1];
     int hi = mend;
     const int target = item_offset + j_begin;
     while (lo < hi) {
@@ -174,15 +176,16 @@ topk_merge_kernel(const float *__restrict__ vals, const int32_t *__restrict__ id
 
 template <int D>
 int launch_score(const float *user_emb, const int64_t *users, int n_users, const float *item_emb, int n_items,
-                 int item_offset, const int32_t *mask_rowptr, const int32_t *mask_cols, int k, int n_splits,
-                 float *ws_val, int32_t *ws_idx, cudaStream_t stream) {
+                 int item_offset, const int32_t *mask_rowptr, const int32_t *mask_cols, int mask_by_user, int k,
+                 int n_splits, float *ws_val, int32_t *ws_idx, cudaStream_t stream) {
   const size_t smem = (size_t)kItemTile * D * sizeof(float) + (size_t)k * kUsers * 8;
   MMREC_REQUIRE(smem <= 227 * 1024, MMREC_E_BADARG, "score_mask_topk: k=%d needs %zu B of shared memory", k, smem);
   MMREC_CUDA(cudaFuncSetAttribute(score_topk_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int items_per_split = ((n_items + n_splits - 1) / n_splits + kItemTile - 1) / kItemTile * kItemTile;
   dim3 grid((n_users + kUsers - 1) / kUsers, n_splits);
   score_topk_kernel<D><<<grid, kUsers, smem, stream>>>(user_emb, users, n_users, item_emb, n_items, item_offset,
-                                                      mask_rowptr, mask_cols, k, items_per_split, ws_val, ws_idx);
+                                                      mask_rowptr, mask_cols, mask_by_user, k, items_per_split,
+                                                      ws_val, ws_idx);
   MMREC_CHECK_LAUNCH("score_topk_kernel");
   return MMREC_OK;
 }
@@ -191,8 +194,8 @@ int launch_score(const float *user_emb, const int64_t *users, int n_users, const
 
 int score_topk_tc_dispatch(const float *user_emb, const int64_t *users, int n_users, const float *item_emb,
                            int n_items, int item_offset, int d, const int32_t *mask_rowptr,
-                           const int32_t *mask_cols, int k, int n_splits, float *ws_val, int32_t *ws_idx,
-                           cudaStream_t stream);   // score_topk_tc.cu
+                           const int32_t *mask_cols, int mask_by_user, int k, int n_splits, float *ws_val,
+                           int32_t *ws_idx, cudaStream_t stream);   // score_topk_tc.cu
 }  // namespace mmrec
 
 using namespace mmrec;
@@ -215,8 +218,8 @@ extern "C" int mmrec_topk_merge(const float *vals, const int32_t *idx, int32_t n
   return MMREC_OK;
 }
 
-static int score_mask_topk(bool allow_tc, const float *user_emb, const int64_t *users, int32_t n_users,
-                           const float *item_emb, int32_t n_items, int32_t item_offset, int32_t d,
+static int score_mask_topk(bool allow_tc, bool mask_by_user, const float *user_emb, const int64_t *users,
+                           int32_t n_users, const float *item_emb, int32_t n_items, int32_t item_offset, int32_t d,
                            const int32_t *mask_rowptr, const int32_t *mask_cols, int32_t k,
                            int32_t n_splits, float *ws_val, int32_t *ws_idx, float *out_val,
                            int64_t *out_idx, void *stream_) {
@@ -232,15 +235,15 @@ static int score_mask_topk(bool allow_tc, const float *user_emb, const int64_t *
   int rc = 1;
   if (allow_tc)      // tcgen05 path (d = 32 / 64); 1 = not covered -> SIMT kernel below
     rc = score_topk_tc_dispatch(user_emb, users, n_users, item_emb, n_items, item_offset, d, mask_rowptr, mask_cols,
-                                k, n_splits, ws_val, ws_idx, stream);
+                                mask_by_user, k, n_splits, ws_val, ws_idx, stream);
   if (rc < 0) return rc;
   if (rc == 1) switch (d) {
     case 32: rc = launch_score<32>(user_emb, users, n_users, item_emb, n_items, item_offset, mask_rowptr, mask_cols,
-                                   k, n_splits, ws_val, ws_idx, stream); break;
+                                   mask_by_user, k, n_splits, ws_val, ws_idx, stream); break;
     case 64: rc = launch_score<64>(user_emb, users, n_users, item_emb, n_items, item_offset, mask_rowptr, mask_cols,
-                                   k, n_splits, ws_val, ws_idx, stream); break;
+                                   mask_by_user, k, n_splits, ws_val, ws_idx, stream); break;
     case 128: rc = launch_score<128>(user_emb, users, n_users, item_emb, n_items, item_offset, mask_rowptr,
-                                     mask_cols, k, n_splits, ws_val, ws_idx, stream); break;
+                                     mask_cols, mask_by_user, k, n_splits, ws_val, ws_idx, stream); break;
     default:
       set_error("score_mask_topk: unsupported d=%d (32, 64, 128)", d);
       return MMREC_E_BADARG;
@@ -254,8 +257,17 @@ extern "C" int mmrec_score_mask_topk_f32(const float *user_emb, const int64_t *u
                                          const int32_t *mask_rowptr, const int32_t *mask_cols, int32_t k,
                                          int32_t n_splits, float *ws_val, int32_t *ws_idx, float *out_val,
                                          int64_t *out_idx, void *stream) {
-  return score_mask_topk(true, user_emb, users, n_users, item_emb, n_items, item_offset, d, mask_rowptr, mask_cols, k,
-                         n_splits, ws_val, ws_idx, out_val, out_idx, stream);
+  return score_mask_topk(true, false, user_emb, users, n_users, item_emb, n_items, item_offset, d, mask_rowptr,
+                         mask_cols, k, n_splits, ws_val, ws_idx, out_val, out_idx, stream);
+}
+
+extern "C" int mmrec_score_mask_topk_rows_f32(const float *user_emb, const int64_t *users, int32_t n_users,
+                                              const float *item_emb, int32_t n_items, int32_t item_offset,
+                                              int32_t d, const int32_t *mask_rowptr, const int32_t *mask_cols,
+                                              int32_t k, int32_t n_splits, float *ws_val, int32_t *ws_idx,
+                                              float *out_val, int64_t *out_idx, void *stream) {
+  return score_mask_topk(true, true, user_emb, users, n_users, item_emb, n_items, item_offset, d, mask_rowptr,
+                         mask_cols, k, n_splits, ws_val, ws_idx, out_val, out_idx, stream);
 }
 
 extern "C" int mmrec_score_mask_topk_simt_f32(const float *user_emb, const int64_t *users, int32_t n_users,
@@ -263,6 +275,6 @@ extern "C" int mmrec_score_mask_topk_simt_f32(const float *user_emb, const int64
                                               int32_t d, const int32_t *mask_rowptr, const int32_t *mask_cols,
                                               int32_t k, int32_t n_splits, float *ws_val, int32_t *ws_idx,
                                               float *out_val, int64_t *out_idx, void *stream) {
-  return score_mask_topk(false, user_emb, users, n_users, item_emb, n_items, item_offset, d, mask_rowptr, mask_cols,
-                         k, n_splits, ws_val, ws_idx, out_val, out_idx, stream);
+  return score_mask_topk(false, false, user_emb, users, n_users, item_emb, n_items, item_offset, d, mask_rowptr,
+                         mask_cols, k, n_splits, ws_val, ws_idx, out_val, out_idx, stream);
 }

@@ -1,5 +1,6 @@
 // Full-rank scoring on the 5th-generation tensor cores, fused with train-item masking and a
-// per-user top-K (K8/K9/K10): the tcgen05 path behind mmrec_score_mask_topk_f32 for d = 32 / 64 / 128.
+// per-user top-K (K8/K9/K10): the tcgen05 path behind mmrec_score_mask_topk_f32 and
+// mmrec_score_mask_topk_rows_f32 for d = 32 / 64 / 128.
 //
 // One CTA owns 128 users (the M = 128 rows of the MMA = the 128 TMEM lanes) and walks its item
 // range in tiles of 64 items. Warp roles:
@@ -118,8 +119,9 @@ template <int D, bool A_TMEM>
 __global__ void __launch_bounds__(kThreadsTC, 1)
 score_topk_tc_kernel(const float *__restrict__ user_emb, const int64_t *__restrict__ users, int n_users,
                      const float *__restrict__ item_emb, int n_items, int item_offset,
-                     const int32_t *__restrict__ mask_rowptr, const int32_t *__restrict__ mask_cols, int k,
-                     int items_per_split, float *__restrict__ ws_val, int32_t *__restrict__ ws_idx, int pend_cap,
+                     const int32_t *__restrict__ mask_rowptr, const int32_t *__restrict__ mask_cols,
+                     int mask_by_user, int k, int items_per_split, float *__restrict__ ws_val,
+                     int32_t *__restrict__ ws_idx, int pend_cap,
                      int dbg) {
   using C = Cfg<D, A_TMEM>;
   static_assert(!A_TMEM || kAcc * kTileN + 2 * D <= 512, "user tile does not fit beside the accumulators");
@@ -276,8 +278,9 @@ score_topk_tc_kernel(const float *__restrict__ user_emb, const int64_t *__restri
     // =============================== epilogue: mask + top-K ==================================
     int mp = 0, mend = 0, next_masked = INT_MAX;
     if (live && mask_rowptr != nullptr) {
-      int lo = mask_rowptr[b_user];
-      mend = mask_rowptr[b_user + 1];
+      const int mrow = mask_by_user ? (int)users[b_user] : b_user;   // batch entry, or the user's own row
+      int lo = mask_rowptr[mrow];
+      mend = mask_rowptr[mrow + 1];
       int hi = mend;
       const int target = item_offset + j_begin;
       while (lo < hi) {
@@ -408,8 +411,8 @@ inline bool a_tmem_64() {   // A/B switch for d <= 64 (d = 128 always keeps its 
 
 template <int D, bool A_TMEM>
 int launch_tc(const float *user_emb, const int64_t *users, int n_users, const float *item_emb, int n_items,
-              int item_offset, const int32_t *mask_rowptr, const int32_t *mask_cols, int k, int n_splits,
-              float *ws_val, int32_t *ws_idx, cudaStream_t stream) {
+              int item_offset, const int32_t *mask_rowptr, const int32_t *mask_cols, int mask_by_user, int k,
+              int n_splits, float *ws_val, int32_t *ws_idx, cudaStream_t stream) {
   using C = Cfg<D, A_TMEM>;
   const size_t fixed = 1024 + C::OFF_HEAP + (size_t)k * kTileM * 8 + (2 * C::STAGES + 2 * kAcc) * 8 + 16;
   const size_t cap = 227 * 1024;
@@ -420,7 +423,7 @@ int launch_tc(const float *user_emb, const int64_t *users, int n_users, const fl
   const int items_per_split = ((n_items + n_splits - 1) / n_splits + kTileN - 1) / kTileN * kTileN;
   dim3 grid((n_users + kTileM - 1) / kTileM, n_splits);
   score_topk_tc_kernel<D, A_TMEM><<<grid, kThreadsTC, smem, stream>>>(user_emb, users, n_users, item_emb, n_items,
-                                                              item_offset, mask_rowptr, mask_cols, k,
+                                                              item_offset, mask_rowptr, mask_cols, mask_by_user, k,
                                                               items_per_split, ws_val, ws_idx, pend_cap,
                                                               dbg_mode());
   MMREC_CHECK_LAUNCH("score_topk_tc_kernel");
@@ -429,13 +432,13 @@ int launch_tc(const float *user_emb, const int64_t *users, int n_users, const fl
 
 }  // namespace
 
-// Called by mmrec_score_mask_topk_f32 (score_topk.cu). Returns 1 if d is not covered here.
+// Called by mmrec_score_mask_topk_f32 / _rows_f32 (score_topk.cu). Returns 1 if d is not covered here.
 int score_topk_tc_dispatch(const float *user_emb, const int64_t *users, int n_users, const float *item_emb,
                            int n_items, int item_offset, int d, const int32_t *mask_rowptr,
-                           const int32_t *mask_cols, int k, int n_splits, float *ws_val, int32_t *ws_idx,
-                           cudaStream_t stream) {
+                           const int32_t *mask_cols, int mask_by_user, int k, int n_splits, float *ws_val,
+                           int32_t *ws_idx, cudaStream_t stream) {
 #define MMREC_TC(D_, T_) launch_tc<D_, T_>(user_emb, users, n_users, item_emb, n_items, item_offset, mask_rowptr, \
-                                            mask_cols, k, n_splits, ws_val, ws_idx, stream)
+                                            mask_cols, mask_by_user, k, n_splits, ws_val, ws_idx, stream)
   switch (d) {
     case 32: return MMREC_TC(32, false);
     case 64: return a_tmem_64() ? MMREC_TC(64, true) : MMREC_TC(64, false);

@@ -111,6 +111,8 @@ SIGNATURES = {
                                             _p, _p, _p, _p, _p]),
     "mmrec_score_mask_topk_simt_f32": (C.c_int, [_p, _p, _i32, _p, _i32, _i32, _i32, _p, _p, _i32, _i32,
                                                  _p, _p, _p, _p, _p]),
+    "mmrec_score_mask_topk_rows_f32": (C.c_int, [_p, _p, _i32, _p, _i32, _i32, _i32, _p, _p, _i32, _i32,
+                                                 _p, _p, _p, _p, _p]),
     "mmrec_topk_metrics_workspace_bytes": (_sz, [_i32]),
     "mmrec_topk_metrics_f64": (C.c_int, [_p, _i32, _i32, _p, _p, _p, _p, _p, _p, _p, _p]),
     "mmrec_topk_merge": (C.c_int, [_p, _p, _i32, _i32, _i32, _p, _p, _p]),

@@ -1362,6 +1362,33 @@ def score_mask_topk(user_emb, users, item_emb, k, mask_rowptr=None, mask_cols=No
 
 
 @torch.no_grad()
+def score_mask_topk_rows(user_emb, users, item_emb, k, mask_rowptr, mask_cols, item_offset=0, n_splits=None,
+                         return_scores=False):
+    """score_mask_topk with the mask as a CSR over the rows of `user_emb` (mmrec_score_mask_topk_rows_f32):
+    the mask of entry b is row users[b] of (mask_rowptr int32 [user_emb.shape[0] + 1], mask_cols int32,
+    ascending global item ids inside each row), e.g. a rank's training CSR; no per-batch mask is built."""
+    user_emb, item_emb = _f32c(user_emb), _f32c(item_emb)
+    lib.require_cuda(user_emb, item_emb, users, mask_rowptr, mask_cols)
+    if mask_rowptr.dtype != torch.int32 or mask_cols.dtype != torch.int32:
+        raise RuntimeError("score_mask_topk_rows: the mask CSR must be int32")
+    if mask_rowptr.numel() != user_emb.shape[0] + 1:
+        raise RuntimeError(f"score_mask_topk_rows: mask_rowptr has {mask_rowptr.numel()} entries, the user table "
+                           f"{user_emb.shape[0]} rows")
+    n, n_items, d = users.numel(), item_emb.shape[0], item_emb.shape[1]
+    _check_ids(users, user_emb.shape[0], "score_mask_topk_rows users")
+    dev = user_emb.device
+    S = n_splits or choose_splits(n, n_items)
+    ws_val = torch.empty(S, n, k, dtype=torch.float32, device=dev)
+    ws_idx = torch.empty(S, n, k, dtype=torch.int32, device=dev)
+    out_val = torch.empty(n, k, dtype=torch.float32, device=dev)
+    out_idx = torch.empty(n, k, dtype=torch.int64, device=dev)
+    lib.call("mmrec_score_mask_topk_rows_f32", lib.ptr(user_emb), lib.ptr(users.contiguous()), n, lib.ptr(item_emb),
+             n_items, item_offset, d, lib.ptr(mask_rowptr.contiguous()), lib.ptr(mask_cols.contiguous()), k, S,
+             lib.ptr(ws_val), lib.ptr(ws_idx), lib.ptr(out_val), lib.ptr(out_idx), lib.stream())
+    return (out_idx, out_val) if return_scores else out_idx
+
+
+@torch.no_grad()
 def topk_merge(vals, idx):
     """K-way merge of [L, n, k] descending lists (ties -> lower id)."""
     L, n, k = vals.shape

@@ -20,6 +20,11 @@ torch.distributed (NCCL over NVLink/NVSwitch on the B200 box, gloo in the CPU te
 * Evaluation: items are cut into P equal ranges; every rank runs the fused score + mask + top-K
   kernel on its item slice (global ids via `item_offset`), the [n, K] (score, id) lists are
   all-gathered and merged with `mmrec_topk_merge` (same tie rule: lower id first).
+* Evaluation of the user-sharded LightGCN (`ShardedEvalData`, `ShardedLightGCN.eval_metric_sums`):
+  after the propagation a rank holds the whole item table, its users' rows, their training edges
+  (the mask, `sb.R`) and their held-out edges (the ground truth), so it scores only its own users,
+  with the mask rows looked up by user id in `sb.R` (mmrec_score_mask_topk_rows_f32). The only
+  collective of a pass besides the propagation is one all-reduce of the [5, K] metric sums.
 """
 from __future__ import annotations
 
@@ -524,11 +529,16 @@ class ShardedLightGCN(torch.nn.Module):
     `user_emb` / `item_emb`: initial tables (this rank's user rows, all item rows); default: xavier
     uniform per table, from fixed seeded 1M-row blocks (the same values at every world size).
     `spmm_fn` / `loss_fns` = (fwd, bwd) replace the CUDA operators (ops.lightgcn_loss_fwd / _bwd
-    signatures), e.g. by float64 CPU arithmetic in tests."""
+    signatures), e.g. by float64 CPU arithmetic in tests; so does `eval_fns` = (topk, metric_sums)
+    for the evaluation (signatures of _topk_rows_cuda and ops.topk_metric_sums).
+
+    Evaluation (`eval_metric_sums`, driven by trainer.Trainer.evaluate with a ShardedEvalData): the
+    forward runs once per pass, cached in eval mode and dropped by train(); each rank scores its own
+    users against the item table with its training CSR `sb.R` as the mask."""
 
     def __init__(self, sb: ShardedBipartite, embedding_size=64, n_layers=4, reg_weight=1e-2, group=None,
                  user_emb=None, item_emb=None, seed=2024, chunks=4, gamma=1e-10, spmm_fn=_spmm_cuda, loss_fns=None,
-                 device=None):
+                 device=None, eval_fns=None):
         super().__init__()
         self.sb, self.group, self.n_layers, self.reg_weight = sb, group, int(n_layers), float(reg_weight)
         self.chunks, self.gamma, self.spmm_fn = chunks, float(gamma), spmm_fn
@@ -547,6 +557,19 @@ class ShardedLightGCN(torch.nn.Module):
         self.embedding_dict["item_emb"].register_post_accumulate_grad_hook(self._finish_item_grad)
         self._pending_item_reg = None
         self.timing = None            # dict: CUDA-event spans per phase (scripts/sharded_train.py)
+        self.eval_fns = eval_fns or (_topk_rows_cuda, ops.topk_metric_sums)
+        self._eval_cache = None
+        self._mask = None
+
+    def train(self, mode=True):
+        self._eval_cache = None
+        return super().train(mode)
+
+    def pre_epoch_processing(self):
+        pass
+
+    def post_epoch_processing(self):
+        pass
 
     def forward(self):
         """-> (this rank's rows of the final user table, the final item table)."""
@@ -591,6 +614,103 @@ class ShardedLightGCN(torch.nn.Module):
         """Top-k item ids (unmasked) for GLOBAL user ids `users`, the same on every rank."""
         uo, io = self.forward()
         return bipartite_score_topk(self.sb, uo, io, users, k, group=self.group)
+
+    @torch.no_grad()
+    def restore_embeddings(self):
+        """(this rank's final user rows, the final item table) of the evaluation forward: computed
+        once per evaluation pass in eval mode (its L item-table all-reduces run on every rank)."""
+        if self.training or self._eval_cache is None:
+            uo, io = self.forward()
+            if self.training:
+                return uo, io
+            self._eval_cache = (uo.contiguous(), io.contiguous())
+        return self._eval_cache
+
+    def _mask_csr(self):
+        """This rank's training CSR as the evaluation mask: (row_ptr, col_idx, col_offset). The
+        kernels walk a mask row with an ascending cursor, so the columns are checked to ascend
+        strictly within every row (once)."""
+        if self._mask is None:
+            R = self.sb.R
+            rp = R.row_ptr
+            a, b = int(rp[0]), int(rp[-1])
+            cols = R.col_idx[a:b]
+            if cols.numel() > 1:
+                up = cols[1:] > cols[:-1]
+                starts = rp[1:-1].to(torch.int64) - a                 # where a row begins, the order may restart
+                up[starts[(starts > 0) & (starts < cols.numel())] - 1] = True
+                if not bool(up.all()):
+                    raise ValueError("ShardedLightGCN: the training CSR's columns must ascend within each row")
+            self._mask = (rp, R.col_idx, R.col_offset)
+        return self._mask
+
+    @torch.no_grad()
+    def eval_topk(self, users, k):
+        """Top-k item ids, training items masked, for LOCAL user ids `users` of this rank, from the
+        evaluation forward. No collective besides that forward's."""
+        uo, io = self.restore_embeddings()
+        rp, cols, off = self._mask_csr()
+        # a CSR whose columns carry an offset (a view of the full graph's user rows) masks with the
+        # offset ids: score them under those ids and map back
+        ids = self.eval_fns[0](uo, users, io, k, rp, cols, off)
+        return ids - off if off else ids
+
+    @torch.no_grad()
+    def eval_metric_sums(self, eval_data, k):
+        """This rank's [5, k] float64 metric sums (ops.topk_metric_sums rows) over its evaluated
+        users `eval_data` (a ShardedEvalData), scored `eval_data.step` users at a time. Every rank
+        must call it: the evaluation forward has collectives. Trainer.evaluate reduces the sums."""
+        uo, io = self.restore_embeddings()
+        rowptr, items = eval_data.gt_csr()
+        n = eval_data.eval_u.numel()
+        sums = torch.zeros(5, k, dtype=torch.float64, device=io.device)
+        for a in range(0, n, eval_data.step):
+            b = min(n, a + eval_data.step)
+            ids = self.eval_topk(eval_data.eval_u[a:b], k)
+            sums += self.eval_fns[1](ids, rowptr[a:b + 1], items)
+        return sums
+
+
+def _topk_rows_cuda(user_emb, users, item_emb, k, mask_rowptr, mask_cols, item_offset):
+    return ops.score_mask_topk_rows(user_emb, users, item_emb, k, mask_rowptr, mask_cols, item_offset=item_offset)
+
+
+class ShardedEvalData:
+    """One rank's share of a held-out split (valid or test) for ShardedLightGCN's evaluation, built
+    on the device from this rank's held-out edges (`users`: global ids in [sb.lo, sb.hi); `items`):
+    * `eval_u`: LOCAL ids of the rank's users with at least one held-out edge, ascending (int64);
+    * `gt_csr()`: their ground truth as EvalDataLoader.gt_csr gives it (int32 row pointers,
+      ascending int32 item ids);
+    * `n_users_global` / `total_pos`: evaluated users and held-out interactions over the whole
+      group (one all-reduce here), the denominators of TopKEvaluator's metrics;
+    * `reduce_metric_sums`: sums a rank's [5, K] metric sums over the group, so every rank forms the
+      same result dict (and makes the same early-stopping decision in Trainer.fit).
+    `batch_users`: evaluated users per scoring launch (bounds the [n, K] workspaces)."""
+
+    def __init__(self, sb: ShardedBipartite, users, items, group=None, batch_users=1 << 17):
+        users = users.to(torch.int64) - sb.lo
+        items = items.to(torch.int64)
+        if users.numel() and (int(users.min()) < 0 or int(users.max()) >= sb.hi - sb.lo):
+            raise ValueError("ShardedEvalData: held-out edges of users this rank does not own")
+        key = torch.sort(users * sb.I + items)[0]
+        self.eval_u, counts = torch.unique_consecutive(key // sb.I, return_counts=True)
+        rowptr = torch.zeros(self.eval_u.numel() + 1, dtype=torch.int64, device=key.device)
+        rowptr[1:] = torch.cumsum(counts, 0)
+        self._gt = (rowptr.to(torch.int32), (key % sb.I).to(torch.int32))
+        cnt = torch.tensor([self.eval_u.numel(), key.numel()], dtype=torch.int64, device=key.device)
+        if sb.world > 1:
+            dist.all_reduce(cnt, group=group)
+        self.n_users_global, self.total_pos = int(cnt[0]), float(cnt[1])
+        self.world, self.group, self.step = sb.world, group, int(batch_users)
+
+    def gt_csr(self):
+        return self._gt
+
+    def reduce_metric_sums(self, sums):
+        if self.world > 1:
+            sums = sums.clone()
+            dist.all_reduce(sums, group=self.group)
+        return sums
 
 
 # ------------------------------------------------------------------ item-range sharded modality tables

@@ -11,6 +11,9 @@ so every benchmark and parity test runs on graphs generated here (SURVEY.md sect
   random permutation;
 * x_label in {0,1,2} w.p. 0.8/0.1/0.1, each user's first row forced to 0 so every evaluated
   user has training rows (dataloader.py:386 `get_group`).
+
+Config 5's scaled graph is generated on the device (`make_scaled_edges`), and its held-out split
+(`scaled_edge_labels`) follows the same rules with a hash per edge instead of a sequential draw.
 """
 from __future__ import annotations
 
@@ -180,3 +183,53 @@ def make_scaled_edges(device, n_users, n_items, n_edges, seed=2024, user_range=N
         z = torch.zeros(0, dtype=torch.int64, device=device)
         return z, z
     return torch.cat(us), torch.cat(its)
+
+
+def _s64(c):
+    """A 64-bit constant as the int64 with the same bits."""
+    return c - (1 << 64) if c >= 1 << 63 else c
+
+
+def _mix64(x):
+    """splitmix64's finaliser on an int64 tensor: wrapping products, logical right shifts."""
+    x = x ^ ((x >> 30) & ((1 << 34) - 1))
+    x = x * _s64(0xBF58476D1CE4E5B9)
+    x = x ^ ((x >> 27) & ((1 << 37) - 1))
+    x = x * _s64(0x94D049BB133111EB)
+    return x ^ ((x >> 31) & ((1 << 33) - 1))
+
+
+def _mix64_int(x):
+    """_mix64 on one Python int (the seed's salt)."""
+    m = (1 << 64) - 1
+    x &= m
+    x ^= x >> 30
+    x = (x * 0xBF58476D1CE4E5B9) & m
+    x ^= x >> 27
+    x = (x * 0x94D049BB133111EB) & m
+    return _s64(x ^ (x >> 31))
+
+
+SPLIT_P = (0.8, 0.1, 0.1)
+
+
+def scaled_edge_labels(users, items, seed=2024):
+    """Held-out split of make_scaled_edges' edges: int64 labels 0 / 1 / 2 (train / valid / test)
+    with probabilities 0.8 / 0.1 / 0.1, as make_interactions draws them for the small shapes; each
+    user's first edge (its lowest item id) is train, so every evaluated user has training rows.
+
+    An edge's label is a counter-based hash of (seed, user, item) (splitmix64's finaliser), not a
+    draw from a sequential stream: a rank that labels only its own users' edges gets exactly the
+    labels the one-rank call gives them, at any world size. `users` / `items` must be sorted by
+    (user, item), as make_scaled_edges returns them, and hold whole users (a user range)."""
+    import torch
+    u, i = users.to(torch.int64), items.to(torch.int64)
+    salt = _mix64_int(int(seed) ^ 0x5851F42D4C957F2D)
+    r = (_mix64((u << 32) + i + salt) >> 40) & ((1 << 24) - 1)          # top 24 bits: uniform in [0, 2^24)
+    t1, t2 = round(SPLIT_P[0] * (1 << 24)), round((SPLIT_P[0] + SPLIT_P[1]) * (1 << 24))
+    labels = (r >= t1).to(torch.int64) + (r >= t2).to(torch.int64)
+    if u.numel():
+        first = torch.ones_like(u, dtype=torch.bool)
+        first[1:] = u[1:] != u[:-1]
+        labels[first] = 0
+    return labels

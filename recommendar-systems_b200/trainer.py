@@ -128,11 +128,20 @@ class TopKEvaluator:
                 out["{}@{}".format(metric, k)] = round(value[k - 1], 4)
         return out
 
+    def evaluate_sums(self, sums, eval_data):
+        """The result dict of a user-sharded evaluation (parallel.ShardedEvalData): `sums` are this
+        rank's [5, K] metric sums; they are summed over the evaluation data's process group and
+        divided by its global counts, so every rank returns the same dict."""
+        sums = eval_data.reduce_metric_sums(sums)
+        return self.result_from_sums(sums, eval_data.n_users_global, eval_data)
+
     def _metrics_from_sums(self, sums, n, eval_data):
         sums = sums.cpu().numpy()
-        if getattr(eval_data, "_total_pos", None) is None:
-            eval_data._total_pos = float(np.asarray(eval_data.get_eval_len_list(), dtype=np.int64).sum())
-        total_pos = eval_data._total_pos
+        total_pos = getattr(eval_data, "total_pos", None)        # global count of sharded evaluation data
+        if total_pos is None:
+            if getattr(eval_data, "_total_pos", None) is None:
+                eval_data._total_pos = float(np.asarray(eval_data.get_eval_len_list(), dtype=np.int64).sum())
+            total_pos = eval_data._total_pos
         rows = {"recall": sums[0] / n, "recall2": sums[1] / total_pos, "precision": sums[2] / n,
                 "ndcg": sums[3] / n, "map": sums[4] / n}
         return np.stack([rows[m] for m in self.metrics], axis=0)
@@ -558,7 +567,14 @@ class Trainer:
         """trainer.py:509-528. On CUDA the whole pass -- evaluation forward, fused score + mask +
         top-K, device metrics -- is captured in a CUDA graph the second time a loader is evaluated
         and replayed afterwards (parameters are read in place, so replays see the current model);
-        one [5, K] float64 copy comes back to the host."""
+        one [5, K] float64 copy comes back to the host.
+        User-sharded evaluation data (parallel.ShardedEvalData, reduce_metric_sums): every rank scores
+        its own users (model.eval_metric_sums) and the sums are reduced over the group; eager, the
+        pass has NCCL calls."""
+        if hasattr(eval_data, "reduce_metric_sums"):
+            self.model.eval()
+            sums = self.model.eval_metric_sums(eval_data, max(self.config["topk"]))
+            return self.evaluator.evaluate_sums(sums, eval_data)
         if not self.use_eval_graph or not hasattr(eval_data, "gt_csr") or not eval_data.eval_u.is_cuda:
             return self.evaluator.evaluate(self.evaluate_topk(eval_data), eval_data, is_test=is_test, idx=idx)
         key = (id(eval_data), id(self.model))
