@@ -110,6 +110,20 @@ int mmrec_spmm_csr_ex_f32(const int32_t *row_ptr, const int32_t *col_idx, const 
                        int32_t *counters, float *scratch, int32_t col_offset, const float *X,
                        int32_t d, float *Y, const float *acc_in, float *acc_out, float acc_scale,
                        const float *cos_ref, float *cos_w, float *Y_pre, int32_t flags, void *stream);
+/* The operator of mmrec_spmm_csr_ex_f32 on a bf16 operand: X is bf16 (raw bits, [n_cols, d],
+ * row-major), widened exactly in registers; every product and sum is fp32, in the order of the
+ * fp32 kernel (same task list, scratch and counters), so Y / acc_out equal what
+ * mmrec_spmm_csr_ex_f32 gives on X converted to float32, bit for bit. Y16 (optional, bf16 bits
+ * [n_rows, d]) receives y rounded to nearest even -- written by the task that finishes the row --
+ * so a caller that needs only the rounded row and the running sum passes Y = NULL.
+ * d must be 32, 64 or 128; flags may be 0 or MMREC_SPMM_NARROW; cos_ref, cos_w and Y_pre must be
+ * NULL (no cosine epilogue). X, Y, Y16, acc_in, acc_out, scratch and tasks 16-byte aligned. */
+int mmrec_spmm_csr_bf16_f32(const int32_t *row_ptr, const int32_t *col_idx, const float *vals,
+                            const int32_t *tasks, int32_t n_tasks, const int32_t *slot_base,
+                            int32_t *counters, float *scratch, int32_t col_offset, const uint16_t *X,
+                            int32_t d, float *Y, uint16_t *Y16, const float *acc_in, float *acc_out,
+                            float acc_scale, const float *cos_ref, float *cos_w, float *Y_pre,
+                            int32_t flags, void *stream);
 
 /* Several independent SpMMs of the same width d in ONE launch (at most 4): the item-item and R
  * propagation of the three modality views (smore.py:291-317, mgcn.py:170-184), which are

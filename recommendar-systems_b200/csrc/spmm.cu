@@ -384,6 +384,190 @@ layergcn_cos_bwd_kernel(const float *__restrict__ dE, const float *__restrict__ 
   }
 }
 
+// ---- bf16 operand, fp32 accumulation (mmrec_spmm_csr_bf16_f32) ------------------------------
+// The task walk of run_task with X stored as bf16: one 16-byte gather is 8 values, so a sub-warp
+// has LANES = d / 8 lanes (CHUNKS 16-byte pieces per lane in the narrow tiling) and lane `lane`
+// owns the elements (q * LANES + lane) * 8 + [0, 8) of a row. The values are widened in registers
+// (exactly: a bf16 is the top half of a float32) and every product and sum is the fp32 arithmetic
+// of the fp32 kernel in the same order (CSR order inside a task, parts in order for a split row,
+// the same epilogue), so the output equals mmrec_spmm_csr_f32's on the widened operand bit for bit.
+struct ProblemBf16 {
+  const int32_t *row_ptr, *col_idx;
+  const float *vals;
+  const int4 *tasks;
+  int n_tasks;
+  const int32_t *slot_base;
+  int32_t *counters;
+  float *scratch;
+  int col_offset;
+  const uint16_t *X;
+  float *Y;
+  uint16_t *Y16;
+  const float *acc_in;
+  float *acc_out;
+  float acc_scale;
+};
+
+__device__ __forceinline__ void fma8_bf16(float4 &lo, float4 &hi, float s, const uint4 &x) {
+  fma4(lo, s, make_float4(__uint_as_float(x.x << 16), __uint_as_float(x.x & 0xffff0000u),
+                          __uint_as_float(x.y << 16), __uint_as_float(x.y & 0xffff0000u)));
+  fma4(hi, s, make_float4(__uint_as_float(x.z << 16), __uint_as_float(x.z & 0xffff0000u),
+                          __uint_as_float(x.w << 16), __uint_as_float(x.w & 0xffff0000u)));
+}
+
+// round to nearest even, two floats -> one word (low half first, the memory order of a bf16 row)
+__device__ __forceinline__ unsigned pack_bf16x2(float a, float b) {
+  unsigned r;
+  asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(b), "f"(a));
+  return r;
+}
+
+template <int LANES, int CHUNKS>
+__device__ __forceinline__ void run_task_bf16(const ProblemBf16 &P, int t, int lane, int d) {
+  constexpr int NIDX = kSeg / LANES;
+  constexpr int DEPTH0 = CHUNKS == 1 ? kDepth : kDepth / 2;
+  constexpr int DEPTH = DEPTH0 < LANES ? DEPTH0 : LANES;   // shuffle sources stay inside the sub-warp
+  const int4 task = __ldg(P.tasks + t);                    // {row, begin, end, slot}
+  const int row = task.x, begin = task.y, end = task.z, n = end - begin;
+  const unsigned mask = group_mask<LANES>();
+  float4 acc[2 * CHUNKS];
+#pragma unroll
+  for (int q = 0; q < 2 * CHUNKS; ++q) acc[q] = make_float4(0.f, 0.f, 0.f, 0.f);
+  int c[NIDX];
+  float v[NIDX];
+#pragma unroll
+  for (int i = 0; i < NIDX; ++i) {
+    const int k = begin + i * LANES + lane;
+    c[i] = 0;
+    v[i] = 0.f;
+    if (k < end) {
+      c[i] = ld_stream_i32(P.col_idx + k) - P.col_offset;
+      v[i] = ld_stream_f32(P.vals + k);
+    }
+  }
+  {
+    // graph constants above, the previous launch's outputs below (see gather_rows / run_task)
+    int probe = 0;
+#pragma unroll
+    for (int i = 0; i < NIDX; ++i) probe |= c[i] | (int)__float_as_uint(v[i]);
+    if (probe != 0x7fc00001) pdl_wait();
+    if (task.w < 0 && P.acc_in) {
+      const size_t o = (size_t)row * d + lane * 8;
+      asm volatile("prefetch.global.L2 [%0];" ::"l"(P.acc_in + o));
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < NIDX; ++i) {
+#pragma unroll
+    for (int j = 0; j < LANES; j += DEPTH) {
+      const int base = i * LANES + j;
+      if (base < n) {
+        int cc[DEPTH];
+        float vv[DEPTH];
+        uint4 x[DEPTH][CHUNKS];
+#pragma unroll
+        for (int s = 0; s < DEPTH; ++s) {
+          cc[s] = __shfl_sync(mask, c[i], j + s, LANES);
+          vv[s] = __shfl_sync(mask, v[i], j + s, LANES);
+        }
+#pragma unroll
+        for (int s = 0; s < DEPTH; ++s)
+#pragma unroll
+          for (int q = 0; q < CHUNKS; ++q)
+            x[s][q] = base + s < n
+                          ? __ldg(reinterpret_cast<const uint4 *>(P.X + (size_t)cc[s] * d + (q * LANES + lane) * 8))
+                          : make_uint4(0u, 0u, 0u, 0u);
+#pragma unroll
+        for (int s = 0; s < DEPTH; ++s)
+#pragma unroll
+          for (int q = 0; q < CHUNKS; ++q) fma8_bf16(acc[2 * q], acc[2 * q + 1], vv[s], x[s][q]);
+      }
+    }
+  }
+  if (task.w >= 0) {
+    // heavy row: publish this part, the last arriver reduces all parts in order
+    const int r0 = P.row_ptr[row];
+    const int n_parts = (P.row_ptr[row + 1] - r0 + kSeg - 1) / kSeg;
+    const int part = (begin - r0) / kSeg;
+    float *base = P.scratch + (size_t)P.slot_base[task.w] * d;
+#pragma unroll
+    for (int q = 0; q < CHUNKS; ++q) {
+      float4 *p = reinterpret_cast<float4 *>(base + (size_t)part * d + (q * LANES + lane) * 8);
+      __stcg(p, acc[2 * q]);
+      __stcg(p + 1, acc[2 * q + 1]);
+    }
+    __threadfence();
+    __syncwarp(mask);
+    int last = 0;
+    if (lane == 0) {
+      last = atomicAdd(P.counters + task.w, 1) == n_parts - 1;
+      if (last) P.counters[task.w] = 0;
+    }
+    last = __shfl_sync(mask, last, 0, LANES);
+    if (!last) return;
+    __threadfence();
+#pragma unroll
+    for (int q = 0; q < 2 * CHUNKS; ++q) acc[q] = make_float4(0.f, 0.f, 0.f, 0.f);
+    constexpr int U = CHUNKS == 1 ? 4 : 2;
+    for (int p = 0; p < n_parts; p += U) {
+      float4 w[U][2 * CHUNKS];
+#pragma unroll
+      for (int u = 0; u < U; ++u)
+#pragma unroll
+        for (int q = 0; q < 2 * CHUNKS; ++q)
+          w[u][q] = p + u < n_parts ? __ldcg(reinterpret_cast<const float4 *>(
+                                          base + (size_t)(p + u) * d + (q / 2 * LANES + lane) * 8 + (q % 2) * 4))
+                                    : make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+      for (int u = 0; u < U; ++u)
+#pragma unroll
+        for (int q = 0; q < 2 * CHUNKS; ++q) {
+          acc[q].x += w[u][q].x; acc[q].y += w[u][q].y; acc[q].z += w[u][q].z; acc[q].w += w[u][q].w;
+        }
+    }
+  }
+  // epilogue of finish_row (no cosine mode), plus the rounded copy of y
+  const size_t off = (size_t)row * d;
+#pragma unroll
+  for (int q = 0; q < CHUNKS; ++q) {
+    const size_t o = off + (q * LANES + lane) * 8;
+    if (P.Y) {
+      *reinterpret_cast<float4 *>(P.Y + o) = acc[2 * q];
+      *reinterpret_cast<float4 *>(P.Y + o + 4) = acc[2 * q + 1];
+    }
+    if (P.Y16) {
+      const float4 a = acc[2 * q], b = acc[2 * q + 1];
+      *reinterpret_cast<uint4 *>(P.Y16 + o) =
+          make_uint4(pack_bf16x2(a.x, a.y), pack_bf16x2(a.z, a.w), pack_bf16x2(b.x, b.y), pack_bf16x2(b.z, b.w));
+    }
+    if (P.acc_out) {
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        float4 r = acc[2 * q + h];
+        if (P.acc_in) {
+          const float4 a = *reinterpret_cast<const float4 *>(P.acc_in + o + 4 * h);
+          r.x += a.x; r.y += a.y; r.z += a.z; r.w += a.w;
+        }
+        r.x *= P.acc_scale; r.y *= P.acc_scale; r.z *= P.acc_scale; r.w *= P.acc_scale;
+        *reinterpret_cast<float4 *>(P.acc_out + o + 4 * h) = r;
+      }
+    }
+  }
+}
+
+// 4-lane and two-chunk tilings hold 16 indices or 16 accumulators per lane: 3 CTAs (80 registers) keep
+// them from spilling
+template <int LANES, int CHUNKS>
+__global__ void __launch_bounds__(kThreads, CHUNKS == 1 && LANES >= 8 ? 4 : 3)
+spmm_csr_bf16_kernel(const ProblemBf16 P, int d) {
+  constexpr int GROUPS = kThreads / LANES;
+  pdl_trigger();
+  const int lane = threadIdx.x % LANES;
+  const int t = blockIdx.x * GROUPS + threadIdx.x / LANES;
+  if (t >= P.n_tasks) return;
+  run_task_bf16<LANES, CHUNKS>(P, t, lane, d);
+}
+
 // Narrow tiling for graphs of very short rows (the column blocks of graph.ColumnBlockedCSR: a
 // handful of non-zeros per task): half the lanes per task, two float4 per lane -- twice as many
 // tasks in flight per SM for a kernel whose time is the number of dependent round trips per task
@@ -410,6 +594,22 @@ int dispatch_width(int d, F &&f) {
     case 256: return f(std::integral_constant<int, 32>{}, std::integral_constant<int, 2>{});
     default:
       set_error("unsupported embedding width d=%d (supported: 32, 64, 128, 256)", d);
+      return MMREC_E_BADARG;
+  }
+}
+
+// (LANES, CHUNKS) of the bf16 kernel: LANES * CHUNKS * 8 = d; the narrow tiling halves the lanes.
+template <typename F>
+int dispatch_width_bf16(int d, bool narrow, F &&f) {
+  using std::integral_constant;
+  switch (d) {
+    case 32: return f(integral_constant<int, 4>{}, integral_constant<int, 1>{});
+    case 64: return narrow ? f(integral_constant<int, 4>{}, integral_constant<int, 2>{})
+                           : f(integral_constant<int, 8>{}, integral_constant<int, 1>{});
+    case 128: return narrow ? f(integral_constant<int, 8>{}, integral_constant<int, 2>{})
+                            : f(integral_constant<int, 16>{}, integral_constant<int, 1>{});
+    default:
+      set_error("spmm_bf16: unsupported embedding width d=%d (supported: 32, 64, 128)", d);
       return MMREC_E_BADARG;
   }
 }
@@ -464,6 +664,39 @@ extern "C" int mmrec_spmm_csr_ex_f32(const int32_t *row_ptr, const int32_t *col_
                                      const float *cos_ref, float *cos_w, float *Y_pre, int32_t flags, void *stream) {
   return spmm_csr_impl(flags, row_ptr, col_idx, vals, tasks, n_tasks, slot_base, counters, scratch, col_offset, X, d,
                        Y, acc_in, acc_out, acc_scale, cos_ref, cos_w, Y_pre, stream);
+}
+
+extern "C" int mmrec_spmm_csr_bf16_f32(const int32_t *row_ptr, const int32_t *col_idx, const float *vals,
+                                       const int32_t *tasks, int32_t n_tasks, const int32_t *slot_base,
+                                       int32_t *counters, float *scratch, int32_t col_offset, const uint16_t *X,
+                                       int32_t d, float *Y, uint16_t *Y16, const float *acc_in, float *acc_out,
+                                       float acc_scale, const float *cos_ref, float *cos_w, float *Y_pre,
+                                       int32_t flags, void *stream) {
+  MMREC_REQUIRE(row_ptr && col_idx && vals && tasks && X, MMREC_E_BADARG, "spmm_bf16: null input");
+  MMREC_REQUIRE(Y || Y16 || acc_out, MMREC_E_BADARG, "spmm_bf16: no output requested");
+  MMREC_REQUIRE(n_tasks >= 0, MMREC_E_BADARG, "spmm_bf16: bad sizes");
+  MMREC_REQUIRE(!cos_ref && !cos_w && !Y_pre, MMREC_E_BADARG, "spmm_bf16: the cosine epilogue has no bf16 variant");
+  MMREC_REQUIRE(!(flags & ~MMREC_SPMM_NARROW), MMREC_E_BADARG,
+                "spmm_bf16: flags 0x%x not supported (MMREC_SPMM_NARROW only)", flags);
+  MMREC_REQUIRE(aligned16(X) && aligned16(Y) && aligned16(Y16) && aligned16(acc_in) && aligned16(acc_out) &&
+                    aligned16(tasks) && aligned16(scratch),
+                MMREC_E_ALIGN, "spmm_bf16: dense operands and the task list must be 16-byte aligned");
+  const void *x = X;
+  MMREC_REQUIRE(x != Y && x != Y16 && x != acc_out, MMREC_E_BADARG, "spmm_bf16: X must not alias an output");
+  const bool narrow = flags & MMREC_SPMM_NARROW;
+  // the width is checked before the n_tasks == 0 exit, so that a bad d never passes unnoticed
+  return dispatch_width_bf16(d, narrow, [&](auto lanes, auto chunks) {
+    constexpr int L = decltype(lanes)::value, C = decltype(chunks)::value;
+    constexpr int GROUPS = kThreads / L;
+    if (n_tasks == 0) return MMREC_OK;
+    const ProblemBf16 P{row_ptr, col_idx, vals, reinterpret_cast<const int4 *>(tasks), n_tasks, slot_base, counters,
+                        scratch, col_offset, X, Y, Y16, acc_in,
+                        acc_out, acc_scale};
+    const int blocks = (n_tasks + GROUPS - 1) / GROUPS;
+    MMREC_CUDA(launch_pdl(spmm_csr_bf16_kernel<L, C>, blocks, kThreads, 0, (cudaStream_t)stream, P, d));
+    MMREC_CHECK_LAUNCH("spmm_csr_bf16_kernel");
+    return MMREC_OK;
+  });
 }
 
 extern "C" int mmrec_spmm_csr_multi_f32(const MmrecSpmmProblem *problems_host, int32_t n_problems, int32_t d,

@@ -31,6 +31,8 @@ SIGNATURES = {
                                      _f32, _p, _p, _p, _p]),
     "mmrec_spmm_csr_ex_f32": (C.c_int, [_p, _p, _p, _p, _i32, _p, _p, _p, _i32, _p, _i32, _p, _p, _p,
                                         _f32, _p, _p, _p, _i32, _p]),
+    "mmrec_spmm_csr_bf16_f32": (C.c_int, [_p, _p, _p, _p, _i32, _p, _p, _p, _i32, _p, _i32, _p, _p, _p, _p,
+                                          _f32, _p, _p, _p, _i32, _p]),
     "mmrec_spmm_csr_multi_f32": (C.c_int, [_p, _i32, _i32, _p]),
     "mmrec_layergcn_cos_bwd_f32": (C.c_int, [_p, _p, _p, _p, _i32, _i32, _p, _p, _p]),
     "mmrec_bpr_fwd_f32": (C.c_int, [_p, _p, _i32, _p, _p, _p, _i32, _p, _p, _p, _p, _p]),

@@ -52,14 +52,21 @@ _NARROW_ALL = __import__("os").environ.get("MMREC_SPMM_NARROW", "0") == "1"     
 
 
 def spmm_raw(g: CSRGraph, X, Y=None, acc_in=None, acc_out=None, acc_scale=1.0, cos_ref=None,
-             cos_w=None, y_pre=None, narrow=False, stream_policy=None):
+             cos_w=None, y_pre=None, narrow=False, stream_policy=None, y16=None):
     """mmrec_spmm_csr_f32 on already-allocated tensors (no autograd). narrow=True: the tiling for
     graphs of very short rows; stream_policy: L2 eviction hints for operands larger than the cache
-    (default: on when the gathered table exceeds half of L2) -- mmrec_spmm_csr_ex_f32."""
+    (default: on when the gathered table exceeds half of L2) -- mmrec_spmm_csr_ex_f32.
+    A bfloat16 X runs mmrec_spmm_csr_bf16_f32 (fp32 arithmetic, fp32 Y / acc); `y16` (bfloat16
+    [n_rows, d]) then receives y rounded to nearest even."""
     lib.require_cuda(X)
     d = X.shape[1]
     if X.shape[0] < g.n_cols:
         raise RuntimeError(f"spmm: X has {X.shape[0]} rows, graph has {g.n_cols} columns")
+    if X.dtype == torch.bfloat16:
+        _spmm_bf16(g, X, Y, y16, acc_in, acc_out, acc_scale, cos_ref, cos_w, y_pre, narrow, stream_policy)
+        return
+    if X.dtype != torch.float32 or y16 is not None:
+        raise RuntimeError(f"spmm: X must be float32 or bfloat16 (y16 only with bfloat16), got {X.dtype}")
     if stream_policy is None:
         stream_policy = _STREAM_DEFAULT and cos_ref is None and 4 * d * g.n_cols > L2_BYTES // 2
     flags = (SPMM_NARROW if (narrow or _NARROW_ALL) else 0) | (SPMM_STREAM if stream_policy else 0)
@@ -75,6 +82,26 @@ def spmm_raw(g: CSRGraph, X, Y=None, acc_in=None, acc_out=None, acc_scale=1.0, c
              lib.ptr(g.scratch(d)), g.col_offset, lib.ptr(X), d, lib.ptr(Y),
              lib.ptr(acc_in), lib.ptr(acc_out), float(acc_scale), lib.ptr(cos_ref), lib.ptr(cos_w),
              lib.ptr(y_pre), lib.stream())
+
+
+def _spmm_bf16(g, X, Y, y16, acc_in, acc_out, acc_scale, cos_ref, cos_w, y_pre, narrow, stream_policy):
+    d = X.shape[1]
+    if not X.is_contiguous():
+        raise RuntimeError("spmm_bf16: X must be contiguous")
+    for name, t, dt in (("Y", Y, torch.float32), ("y16", y16, torch.bfloat16), ("acc_in", acc_in, torch.float32),
+                        ("acc_out", acc_out, torch.float32)):
+        if t is None:
+            continue
+        lib.require_cuda(t)
+        if t.dtype != dt or tuple(t.shape) != (g.n_rows, d) or not t.is_contiguous():
+            raise RuntimeError(f"spmm_bf16: {name} must be a contiguous {dt} [{g.n_rows}, {d}] tensor, "
+                               f"got {t.dtype} {tuple(t.shape)}")
+    flags = (SPMM_NARROW if (narrow or _NARROW_ALL) else 0) | (SPMM_STREAM if stream_policy else 0)
+    lib.call("mmrec_spmm_csr_bf16_f32", lib.ptr(g.row_ptr), lib.ptr(g.col_idx), lib.ptr(g.vals),
+             lib.ptr(g.tasks), g.n_tasks, lib.ptr(g.slot_base), lib.ptr(g.counters),
+             lib.ptr(g.scratch(d)), g.col_offset, lib.ptr(X), d, lib.ptr(Y), lib.ptr(y16),
+             lib.ptr(acc_in), lib.ptr(acc_out), float(acc_scale), lib.ptr(cos_ref), lib.ptr(cos_w),
+             lib.ptr(y_pre), flags, lib.stream())
 
 
 def spmm_blocked_raw(bg, X, Y):

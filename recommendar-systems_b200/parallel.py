@@ -193,8 +193,16 @@ def sharded_score_topk(user_emb, users, item_emb_local, item_lo, k, mask_rowptr=
 
 
 # ------------------------------------------------------------------ user-partitioned bipartite
-def _spmm_cuda(g, X, Y=None, acc_in=None, acc_out=None, scale=1.0, narrow=False):
-    ops.spmm_raw(g, X, Y=Y, acc_in=acc_in, acc_out=acc_out, acc_scale=scale, narrow=narrow)
+def _spmm_cuda(g, X, Y=None, acc_in=None, acc_out=None, scale=1.0, narrow=False, y16=None):
+    ops.spmm_raw(g, X, Y=Y, acc_in=acc_in, acc_out=acc_out, acc_scale=scale, narrow=narrow, y16=y16)
+
+
+PRECISIONS = ("fp32", "bf16")
+
+
+def _check_precision(precision):
+    if precision not in PRECISIONS:
+        raise ValueError(f"precision must be one of {PRECISIONS}, got {precision!r}")
 
 
 class ShardedBipartite:
@@ -281,7 +289,8 @@ class ShardedBipartite:
 
 @torch.no_grad()
 def bipartite_propagate_mean(sb: ShardedBipartite, Xu_local, Xi, n_layers, group=None, spmm_fn=_spmm_cuda,
-                             chunks=4, timing=None, reduce_items=False, after_first_exchange=None):
+                             chunks=4, timing=None, reduce_items=False, after_first_exchange=None,
+                             precision="fp32"):
     """mean_{l=0..L} A^l X0 for a bipartite graph, users sharded / items replicated.
     Xu_local [hi - lo, d]: this rank's user rows of X0; Xi [I, d]: the item rows (same on every
     rank). Returns (users' rows of this rank, all item rows).
@@ -302,7 +311,18 @@ def bipartite_propagate_mean(sb: ShardedBipartite, Xu_local, Xi, n_layers, group
     (a) of the next layer as well: the compute stream waits for the reduced yi_l only right before
     (b) of layer l + 1. With P ranks (a) + (b) is ~2 nnz / P of gather work per layer against one
     4 I d all-reduce, so the exchange hides completely while it is the shorter of the two.
-    `timing` (dict of lists of (start, end) CUDA events per phase) is filled when given."""
+    `timing` (dict of lists of (start, end) CUDA events per phase) is filled when given.
+
+    precision="bf16": the operand every SpMM gathers from is bfloat16 (half the bytes per gathered
+    row), everything else stays in the dtype of the inputs. Layer 1 gathers Xu_local / Xi rounded
+    once (with reduce_items: the reduced item operand, rounded after its all-reduce); layer l > 1
+    gathers layer l - 1's output rounded to nearest even: the user rows by the SpMM that computes
+    them (`y16`; no full-precision copy is written), the item rows after their all-reduce, from the
+    reduced values (the same on every rank). The running sums add the unrounded layer outputs to
+    the unrounded Xu_local / Xi. `spmm_fn` then receives bfloat16 X and, on the user side, y16=
+    instead of Y=."""
+    _check_precision(precision)
+    lowp = precision == "bf16"
     L = n_layers
     multi = sb.world > 1
     if L == 0:
@@ -315,7 +335,11 @@ def bipartite_propagate_mean(sb: ShardedBipartite, Xu_local, Xi, n_layers, group
     scale = 1.0 / (L + 1)
     acc_u, acc_i = Xu_local, Xi.clone()
     xu, xi = Xu_local.contiguous(), Xi.contiguous()
-    d = xi.shape[1]
+    if lowp:
+        xu = xu.to(torch.bfloat16)
+        if not reduce_items:                                  # else rounded once reduced, in layer 1
+            xi = xi.to(torch.bfloat16)
+    d = acc_i.shape[1]
     blocked = getattr(sb, "Rt_blocked", None)
     parts = sb.rt_chunks(chunks) if blocked is None else None
 
@@ -341,7 +365,7 @@ def bipartite_propagate_mean(sb: ShardedBipartite, Xu_local, Xi, n_layers, group
         pending = (works, None)
     for l in range(1, L + 1):
         last = l == L
-        yi = torch.empty(sb.I, d, dtype=xi.dtype, device=xi.device)
+        yi = torch.empty(sb.I, d, dtype=acc_i.dtype, device=acc_i.device)
         works = []
         ev = mark("rt_spmm")
         if blocked is not None:
@@ -372,10 +396,15 @@ def bipartite_propagate_mean(sb: ShardedBipartite, Xu_local, Xi, n_layers, group
             if pending[1] is not None:
                 acc_i.add_(pending[1])
                 xi = pending[1]
+            if lowp:                                          # round the reduced item rows
+                xi = xi.to(torch.bfloat16)
         yu = None if last else torch.empty_like(xu)
-        acc_new = torch.empty_like(xu)
+        acc_new = torch.empty_like(acc_u if lowp else xu)
         ev = mark("r_spmm")
-        spmm_fn(sb.R, xi, Y=yu, acc_in=acc_u, acc_out=acc_new, scale=scale if last else 1.0)
+        if lowp:
+            spmm_fn(sb.R, xi, acc_in=acc_u, acc_out=acc_new, scale=scale if last else 1.0, y16=yu)
+        else:
+            spmm_fn(sb.R, xi, Y=yu, acc_in=acc_u, acc_out=acc_new, scale=scale if last else 1.0)
         done(ev)
         acc_u = acc_new
         pending = (works, yi)
@@ -428,31 +457,35 @@ class _BipartitePropagateMean(torch.autograd.Function):
     triples it owns) and is summed over the group by the operator's first, overlapped, exchange."""
 
     @staticmethod
-    def forward(ctx, Xu_local, Xi, sb, n_layers, group, spmm_fn, chunks, timing, backward_exchange_hook):
-        ctx.args = (sb, n_layers, group, spmm_fn, chunks, timing, backward_exchange_hook)
+    def forward(ctx, Xu_local, Xi, sb, n_layers, group, spmm_fn, chunks, timing, backward_exchange_hook, precision):
+        ctx.args = (sb, n_layers, group, spmm_fn, chunks, timing, backward_exchange_hook, precision)
         ev = _span(timing, "forward_propagation")
-        out = bipartite_propagate_mean(sb, Xu_local.detach(), Xi.detach(), n_layers, group, spmm_fn, chunks, timing)
+        out = bipartite_propagate_mean(sb, Xu_local.detach(), Xi.detach(), n_layers, group, spmm_fn, chunks, timing,
+                                       precision=precision)
         _end(ev)
         return out
 
     @staticmethod
     def backward(ctx, dU, dI):
-        sb, L, group, spmm_fn, chunks, timing, hook = ctx.args
+        sb, L, group, spmm_fn, chunks, timing, hook, precision = ctx.args
         ev = _span(timing, "backward_propagation")
         gu, gi = bipartite_propagate_mean(sb, dU.contiguous(), dI.contiguous(), L, group, spmm_fn, chunks, timing,
-                                          reduce_items=True, after_first_exchange=hook)
+                                          reduce_items=True, after_first_exchange=hook, precision=precision)
         _end(ev)
-        return gu, gi, None, None, None, None, None, None, None
+        return gu, gi, None, None, None, None, None, None, None, None
 
 
 def bipartite_propagate(sb: ShardedBipartite, Xu_local, Xi, n_layers, group=None, spmm_fn=_spmm_cuda, chunks=4,
-                        timing=None, backward_exchange_hook=None):
+                        timing=None, backward_exchange_hook=None, precision="fp32"):
     """Differentiable bipartite_propagate_mean. Backward exchanges: one chunked all-reduce of the
     partial item gradient, then one per layer as in the forward (1 + L); the returned item
     gradient is the group's total, identical on every rank. `backward_exchange_hook` is the
-    backward's `after_first_exchange` (see bipartite_propagate_mean)."""
+    backward's `after_first_exchange` (see bipartite_propagate_mean). `precision` applies to the
+    forward and to the backward, which runs the same operator (rounding the incoming gradients
+    where the forward rounds the tables; the item gradient after its reduction)."""
+    _check_precision(precision)
     return _BipartitePropagateMean.apply(Xu_local, Xi, sb, n_layers, group, spmm_fn, chunks, timing,
-                                         backward_exchange_hook)
+                                         backward_exchange_hook, precision)
 
 
 def _xavier_rows(n, d, lo, hi, seed, device):
@@ -528,6 +561,9 @@ class ShardedLightGCN(torch.nn.Module):
 
     `user_emb` / `item_emb`: initial tables (this rank's user rows, all item rows); default: xavier
     uniform per table, from fixed seeded 1M-row blocks (the same values at every world size).
+    `precision` ("fp32" or "bf16"): the operand precision of the propagation's SpMMs in the
+    training forward, its backward and the evaluation forward (see bipartite_propagate_mean);
+    parameters, optimizer state, loss and scoring stay float32 either way.
     `spmm_fn` / `loss_fns` = (fwd, bwd) replace the CUDA operators (ops.lightgcn_loss_fwd / _bwd
     signatures), e.g. by float64 CPU arithmetic in tests; so does `eval_fns` = (topk, metric_sums)
     for the evaluation (signatures of _topk_rows_cuda and ops.topk_metric_sums).
@@ -538,8 +574,10 @@ class ShardedLightGCN(torch.nn.Module):
 
     def __init__(self, sb: ShardedBipartite, embedding_size=64, n_layers=4, reg_weight=1e-2, group=None,
                  user_emb=None, item_emb=None, seed=2024, chunks=4, gamma=1e-10, spmm_fn=_spmm_cuda, loss_fns=None,
-                 device=None, eval_fns=None):
+                 device=None, eval_fns=None, precision="fp32"):
         super().__init__()
+        _check_precision(precision)
+        self.precision = precision
         self.sb, self.group, self.n_layers, self.reg_weight = sb, group, int(n_layers), float(reg_weight)
         self.chunks, self.gamma, self.spmm_fn = chunks, float(gamma), spmm_fn
         self.loss_fns = loss_fns or _loss_fns_cuda()
@@ -575,7 +613,8 @@ class ShardedLightGCN(torch.nn.Module):
         """-> (this rank's rows of the final user table, the final item table)."""
         e = self.embedding_dict
         return bipartite_propagate(self.sb, e["user_emb"], e["item_emb"], self.n_layers, self.group, self.spmm_fn,
-                                   self.chunks, self.timing, backward_exchange_hook=self._issue_item_reg)
+                                   self.chunks, self.timing, backward_exchange_hook=self._issue_item_reg,
+                                   precision=self.precision)
 
     def calculate_loss(self, interaction):
         """interaction: this rank's [3, B_p] triples (users as LOCAL row ids, global item ids; B_p

@@ -1,7 +1,7 @@
 """LightGCN trained AND evaluated on config 5's graph (scaled power-law, 10M users x 2M items x ~486M
 interactions, d = 64, 4 layers) with parallel.ShardedLightGCN, one process per GPU:
 
-    python scripts/sharded_fit.py --gpus N [--epochs 2] [--scale 1.0] [--batch 1048576]
+    python scripts/sharded_fit.py --gpus N [--epochs 2] [--scale 1.0] [--batch 1048576] [--precision bf16]
 
 The generated edges are split into train / valid / test (synth.scaled_edge_labels, 0.8 / 0.1 /
 0.1, each user's first edge train); every rank labels only its own users' edges. The normalised
@@ -62,7 +62,7 @@ def worker(rank, world, args):
     valid = par.ShardedEvalData(sb, su[lab == 1], si[lab == 1], batch_users=args.eval_users)
     test = par.ShardedEvalData(sb, su[lab == 2], si[lab == 2], batch_users=args.eval_users)
     del su, si, lab, t
-    model = par.ShardedLightGCN(sb, d, L, 1e-2, chunks=args.chunks)
+    model = par.ShardedLightGCN(sb, d, L, 1e-2, chunks=args.chunks, precision=args.precision)
     cfg = cfgm.Config("LightGCN", "scaled", {"device": torch.device(dev), "cuda_graph": False, "epochs": args.epochs,
                                              "eval_step": 1, "stopping_step": args.stopping_step, "metrics": METRICS,
                                              "topk": TOPK, "valid_metric": "Recall@20"})
@@ -144,7 +144,8 @@ def worker(rank, world, args):
                 "valid_metric": "recall@20", "best_valid_score": best_score, "setup_seconds_rank0": setup_s,
                 "peak_mem_gib_setup_per_rank": [p[0] for p in peaks],
                 "peak_mem_gib_fit_per_rank": [p[1] for p in peaks], "chunks": args.chunks,
-                "rt_block_users": args.rt_block_users, "eval_users_per_launch": args.eval_users,
+                "rt_block_users": args.rt_block_users, "precision": args.precision,
+                "eval_users_per_launch": args.eval_users,
                 "gpu": info, "clocks": clocks}
         bench.emit(line)
     if world > 1:
@@ -161,6 +162,8 @@ def main():
     ap.add_argument("--scale", type=float, default=1.0)
     ap.add_argument("--chunks", type=int, default=4)
     ap.add_argument("--rt-block-users", type=int, default=393216)
+    ap.add_argument("--precision", choices=["fp32", "bf16"], default="fp32",
+                    help="operand precision of the propagation SpMMs (parallel.bipartite_propagate_mean)")
     ap.add_argument("--eval-users", type=int, default=1 << 17)
     args = ap.parse_args()
     if args.gpus == 1:

@@ -1,7 +1,7 @@
 """LightGCN training on config 5's graph (scaled power-law, 10M users x 2M items x ~486M
 interactions, d = 64, 4 layers) with parallel.ShardedLightGCN, one process per GPU:
 
-    python scripts/sharded_train.py --gpus N [--steps 10] [--warmup 3] [--batch 1048576]
+    python scripts/sharded_train.py --gpus N [--steps 10] [--warmup 3] [--batch 1048576] [--precision bf16]
 
 Every rank generates and keeps only its own users' edges (as bench.scaled_block does, including
 the L2-resident user blocks of R^T), draws per-rank batches with data.DeviceTrainLoader and is
@@ -61,7 +61,7 @@ def worker(rank, world, args):
                                                rt_block_users=args.rt_block_users)
     loader = data_m.DeviceTrainLoader(su, si, hi - lo, I, args.batch, seed=999, rank=rank, world=world, user_lo=lo)
     del su, si
-    model = par.ShardedLightGCN(sb, d, L, 1e-2, chunks=args.chunks)
+    model = par.ShardedLightGCN(sb, d, L, 1e-2, chunks=args.chunks, precision=args.precision)
     cfg = cfgm.Config("LightGCN", "scaled", {"device": torch.device(dev), "cuda_graph": False})
     trainer = trm.Trainer(cfg, model)
     torch.cuda.empty_cache()
@@ -139,7 +139,7 @@ def worker(rank, world, args):
                               "is the FusedAdam step",
                 "peak_mem_gib_setup_per_rank": [p[0] for p in peaks],
                 "peak_mem_gib_steps_per_rank": [p[1] for p in peaks], "last_loss": last_loss, "chunks": args.chunks,
-                "rt_block_users": args.rt_block_users, "gpu": info, "clocks": clocks}
+                "rt_block_users": args.rt_block_users, "precision": args.precision, "gpu": info, "clocks": clocks}
         bench.emit(line)
     if world > 1:
         dist.barrier()
@@ -155,6 +155,8 @@ def main():
     ap.add_argument("--scale", type=float, default=1.0)
     ap.add_argument("--chunks", type=int, default=4)
     ap.add_argument("--rt-block-users", type=int, default=393216)
+    ap.add_argument("--precision", choices=["fp32", "bf16"], default="fp32",
+                    help="operand precision of the propagation SpMMs (parallel.bipartite_propagate_mean)")
     args = ap.parse_args()
     if args.gpus == 1:
         worker(0, 1, args)
