@@ -210,7 +210,8 @@ int mmrec_lightgcn_loss_bwd_f32(const float *user_out, const float *item_out, co
  * 2048-row batch fills 148 SMs; dV1_ws/dV2_ws hold n_splits*batch*d floats of partial sums that
  * the scatter kernel adds in split order; mmrec_infonce_splits(batch) is the count that fills
  * the GPU (4 co-resident CTAs per SM). partial (fwd) must hold
- * mmrec_infonce_fwd_workspace_floats(batch) floats; counter is an array of 1 + ceil(batch/64)
+ * mmrec_infonce_fwd_workspace_floats(batch) floats (enough for the mma.sync and the tcgen05
+ * layout at every batch size); counter is an array of 1 + ceil(batch/64)
  * zero-initialised uint32 (self-resetting); batch <= 65472.
  * ---------------------------------------------------------------------------------------- */
 int32_t mmrec_infonce_splits(int32_t batch);

@@ -492,8 +492,10 @@ extern "C" int mmrec_bpr_bwd_f32(const float *user_emb, const float *item_emb, i
 }
 
 extern "C" int32_t mmrec_infonce_splits(int32_t batch) { return infonce_splits(batch); }
+// Enough for both forward layouts: mma.sync pos | ttl_part[splits] | tile_loss, tcgen05 pos | ttl_part[2 * s]
+// with s = infonce_tc_splits(batch, splits) <= max(1, splits / 2), so 2 * s <= max(2, splits).
 extern "C" size_t mmrec_infonce_fwd_workspace_floats(int32_t batch) {
-  return (size_t)(1 + infonce_splits(batch)) * batch + (batch + kTile - 1) / kTile;
+  return (size_t)(1 + max(2, infonce_splits(batch))) * batch + (batch + kTile - 1) / kTile;
 }
 
 extern "C" int mmrec_infonce_fwd_f32(const float *T1, const float *T2, int32_t d, const int64_t *idx,
